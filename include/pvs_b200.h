@@ -33,14 +33,18 @@ extern "C" {
 typedef enum pvs_status {
     PVS_OK = 0,
     PVS_ERR_INVALID_ARG = 1,   /* null pointer, negative size, bad enum */
-    PVS_ERR_UNSUPPORTED_K = 2, /* hidden width outside 1..PVS_MAX_K */
+    PVS_ERR_UNSUPPORTED_K = 2, /* hidden width outside 1..PVS_MAX_K (forward in a
+                                  tensor-core math mode: 1..PVS_MAX_K_TC_FWD) */
     PVS_ERR_TOO_LARGE = 3,     /* one complex does not fit the cell-list smem */
     PVS_ERR_CUDA = 4,          /* a CUDA call failed: pvs_last_cuda_error() */
     PVS_ERR_WORKSPACE = 5,     /* workspace smaller than *_workspace_bytes */
     PVS_ERR_UNSUPPORTED = 6    /* valid request the kernels do not cover yet */
 } pvs_status;
 
-#define PVS_MAX_K 64          /* widest hidden size (--channels) supported */
+#define PVS_MAX_K 64          /* widest hidden size (--channels) every path supports */
+#define PVS_MAX_K_TC_FWD 128  /* widest hidden size of the forward in the tensor-core
+                                 math modes (bf16x3 / fp16x2 / bf16); the backward,
+                                 the stacked training calls and fp32 stop at PVS_MAX_K */
 #define PVS_MAX_EDGE_CLASSES 8
 #define PVS_TILE_EDGES 128    /* edges per work tile (one tcgen05 M=128 tile) */
 #define PVS_TILE_NODES 128    /* node cap per work tile */
@@ -51,6 +55,7 @@ typedef enum pvs_status {
 #define PVS_CAP_BWD_FP32 4u      /* backward kernels                          */
 #define PVS_CAP_FWD_FP16X2 8u    /* PVS_MATH_FP16X2 edge kernel               */
 #define PVS_CAP_CROP 16u         /* K0: pvs_crop_count / pvs_crop_fill        */
+#define PVS_CAP_FWD_WIDE_K 32u   /* forward at 65..PVS_MAX_K_TC_FWD (tcgen05)  */
 
 /* pvs_layer_config.flags -- EGNNLayer.__init__ (egnn_satorras.py:26-46) */
 #define PVS_F_RESIDUAL 0x001u

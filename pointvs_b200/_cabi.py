@@ -29,12 +29,14 @@ F_SOFTMAX_ATTENTION = 0x800
 
 ACT = {'none': 0, 'sigmoid': 1, 'tanh': 2, 'relu': 3, 'silu': 4, 'softplus': 5}
 MATH = {'fp32': 0, 'bf16x3': 1, 'bf16': 2, 'fp16x2': 3}
-MAX_K = 64
+MAX_K = 64            # every path, training included
+MAX_K_TC_FWD = 128    # forward (scoring) in the tensor-core math modes
 TILE_EDGES = 128
 
 CAP_FWD_FP32 = 1
 CAP_FWD_TCGEN05 = 2
 CAP_BWD_FP32 = 4
+CAP_FWD_WIDE_K = 32
 
 _fp = C.c_void_p
 

@@ -20,7 +20,19 @@ import torch
 import yaml
 from torch import nn
 
+from . import _cabi
+
 DEVICE = torch.device('cuda' if torch.cuda.is_available() else 'cpu')
+
+
+def check_trainable_width(k):
+    """The backward kernels cover hidden widths up to _cabi.MAX_K; wider
+    models (up to _cabi.MAX_K_TC_FWD) can be scored but not trained."""
+    if k is not None and int(k) > _cabi.MAX_K:
+        raise NotImplementedError(
+            f'hidden width {k}: training supports --channels up to '
+            f'{_cabi.MAX_K}; models up to {_cabi.MAX_K_TC_FWD} channels can '
+            'only be scored, in a tensor-core math mode')
 
 
 def find_latest_checkpoint(root, model_task=None):
@@ -193,6 +205,7 @@ class PointNeuralNetworkBase(nn.Module):
         a float and raises on NaN at once, as the reference does; sync=False
         returns the loss as a device tensor and leaves the NaN check to the
         caller, so the host can run ahead of the device (N1)."""
+        self._check_trainable()
         loss = self.get_loss(y_true, y_pred)
         arena = self._arena_for_step(loss)
         # from now on the forward passes of this model may take the lean
@@ -263,8 +276,16 @@ class PointNeuralNetworkBase(nn.Module):
             else self.p_epoch
         return init_epoch, time.time()
 
+    def _check_trainable(self):
+        if '_width_checked' not in self.__dict__:     # once per model
+            check_trainable_width(max(
+                (m.hidden_nf for m in self.modules() if hasattr(m, 'hidden_nf')),
+                default=None))
+            self.__dict__['_width_checked'] = True
+
     def train_model(self, data_loader, epochs=1, epoch_end_validation_set=None,
                     top1_on_end=False):
+        self._check_trainable()
         init_epoch, _ = self.training_setup(data_loader, epochs)
         losses, pending, overflow = [], [], []
         for _ in range(init_epoch, epochs):

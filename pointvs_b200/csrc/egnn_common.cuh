@@ -14,10 +14,10 @@ struct EdgeArgs {
     // edge-packed tiles (tcgen05 kernel only): see pvs_graph
     const int32_t *ptile_last, *n_ptiles;
     int n_nodes;
-    float *Mpart;            // [n_ptiles_cap][2][64] partial message sums of split nodes
+    float *Mpart;            // [n_ptiles_cap][2][KP] partial message sums of split nodes
     float *xpart;            // [n_ptiles_cap][2][4]  partial coordinate sums
     // activations
-    const float *P, *Q;      // [N][KP]
+    const float *P, *Q;      // [N][KP], KP = 64 (k <= 64 in the tcgen05 modes) or 128
     const float *x_in;       // [N][3]
     const float *m_prev;     // [E][k] or null
     float *M;                // [N][KP]
@@ -72,5 +72,14 @@ int launch_node_tc(const float *h_in, const float *M, float *h_out, float *natt_
                    const pvs_layer_params *p, int n_nodes, int k, uint32_t flags, int att_act,
                    int mode, cudaStream_t st, int phase = 0, float *V = nullptr,
                    const float *gn_a = nullptr, const float *gn_b = nullptr);
+// the same two stages at 65 <= k <= 128 (egnn_wide_tc.cu): P, Q, M, V at pitch
+// 128; launch_node_pre_tc / launch_node_tc dispatch to them when k > 64
+int launch_wide_node_pre_tc(const float *h, const float *edge_w1, const float *edge_b1, float *P,
+                            float *Q, int n_nodes, int k, int in_e, int perm, int mode,
+                            cudaStream_t st);
+int launch_wide_node_tc(const float *h_in, const float *M, float *h_out, float *natt_out,
+                        const pvs_layer_params *p, int n_nodes, int k, uint32_t flags,
+                        int att_act, int mode, cudaStream_t st, int phase, float *V,
+                        const float *gn_a, const float *gn_b);
 
 }  // namespace pvs

@@ -4,7 +4,8 @@
 // 64x64 contractions (edge_mlp.2 and coord_mlp.0; reference
 // egnn_satorras.py:76-80, 88-96) run as tcgen05.mma tiles:
 //
-//   tile      : 128 dst-sorted edges (UMMA M = 128, cta_group::1), N = 64, K = 64;
+//   tile      : 128 dst-sorted edges (UMMA M = 128, cta_group::1), N = K = KW
+//               (64; 128 for the forward at 64 < k <= 128, see TcCfg);
 //               edge-packed (pvs_build_packed_tiles): tile t = edges
 //               [128 t, 128 t + 128), nodes cut by a tile boundary go through
 //               per-tile partial slots and edge_tile_fixup_kernel
@@ -58,17 +59,31 @@ constexpr int TC_GROUP_THREADS = 128;
 //                costs ~3e-6 on the scores (the fp32 path itself is at 1e-6;
 //                bf16 activations would cost 3e-5) and frees the lo tile.
 enum { TCM_BF16 = 0, TCM_BF16X3 = 1, TCM_FP16X2 = 2 };
-template <int MODE> struct TcCfg {
+// KW = padded hidden width of the tile: 64 (k <= 64) or 128 (65 <= k <= 128,
+// forward only).  At KW = 128 a K-major operand is two SWIZZLE_128B K-blocks of
+// 64 channels, the weights take four times the shared memory and a group
+// needs 128 TMEM columns, so fewer groups fit: bf16x3 128 KB of weight tiles +
+// 64 KB of A tiles per group -> 1 group; fp16x2 128 + 32 -> 2; bf16 64 + 32 -> 4.
+template <int MODE, int KW = 64> struct TcCfg {
     static constexpr bool A_LO = MODE == TCM_BF16X3;      // second activation tile
     static constexpr bool B_LO = MODE != TCM_BF16;        // second weight tile
     static constexpr bool F16 = MODE == TCM_FP16X2;
     static constexpr bool EXACT_SILU = MODE != TCM_BF16;
-    static constexpr int GROUPS = A_LO ? PVS_EXP_GROUPS : 8;
+    static constexpr int GROUPS = KW == 64 ? (A_LO ? PVS_EXP_GROUPS : 8)
+                                           : (A_LO ? 1 : (B_LO ? 2 : 4));
     static constexpr int THREADS = TC_GROUP_THREADS * GROUPS;
+    static constexpr int KB = KW / 64;                    // 64-channel K-blocks
 };
-constexpr int TC_K = 64;          // padded hidden width of the tile
 constexpr uint32_t TC_TMEM_COLS = 512;   // whole TMEM: one CTA per SM
-constexpr uint32_t TC_GROUP_COLS = 64;   // D1 and D2 alias (never live together)
+// a group's TMEM columns: KW (D1 and D2 alias, never live together)
+
+// byte offset of 16-byte chunk `c` (channels 8c..8c+7) of row `r` in a
+// [KW / 64][rows][128 B] tile of K-blocks with `rows` rows each
+template <int KW, int ROWS = TE>
+__device__ __forceinline__ uint32_t swzk(int r, int c) {
+    if constexpr (KW == 64) return swz(r, c);
+    else return (uint32_t)((c >> 3) * (ROWS * 128)) + swz(r, c & 7);
+}
 
 #ifdef PVS_PHASE_PROF
 // Debug build only (scripts/phase_prof.py): cycles each group spends between
@@ -96,19 +111,20 @@ struct TcGroupMisc {
     uint64_t mbar;
 };
 
-template <int MODE>
+template <int MODE, int KW = 64>
 struct __align__(1024) TcSmem {
-    static constexpr int G = TcCfg<MODE>::GROUPS;
-    static constexpr bool X3 = TcCfg<MODE>::A_LO, BLO = TcCfg<MODE>::B_LO;
-    // swizzled bf16 tiles, each 1024-byte aligned (lo tiles only where used)
-    uint8_t A_hi[G][TE * 128];
-    uint8_t A_lo[X3 ? G : 1][X3 ? TE * 128 : 1024];
-    uint8_t W2_hi[TC_K * 128];
-    uint8_t W2_lo[BLO ? TC_K * 128 : 1024];
-    uint8_t Wc1_hi[TC_K * 128];
-    uint8_t Wc1_lo[BLO ? TC_K * 128 : 1024];
-    float b2[64], bc1[64], wc2[64], wa[64], wr[64];
-    float T[PVS_MAX_EDGE_CLASSES][64];
+    static constexpr int G = TcCfg<MODE, KW>::GROUPS, KB = KW / 64;
+    static constexpr bool X3 = TcCfg<MODE, KW>::A_LO, BLO = TcCfg<MODE, KW>::B_LO;
+    // swizzled bf16 tiles, each 1024-byte aligned (lo tiles only where used);
+    // K-block b of a tile starts at b * rows * 128 bytes
+    uint8_t A_hi[G][KB * TE * 128];
+    uint8_t A_lo[X3 ? G : 1][X3 ? KB * TE * 128 : 1024];
+    uint8_t W2_hi[KB * KW * 128];
+    uint8_t W2_lo[BLO ? KB * KW * 128 : 1024];
+    uint8_t Wc1_hi[KB * KW * 128];
+    uint8_t Wc1_lo[BLO ? KB * KW * 128 : 1024];
+    float b2[KW], bc1[KW], wc2[KW], wa[KW], wr[KW];
+    float T[PVS_MAX_EDGE_CLASSES][KW];
     TcGroupMisc grp[G];
     uint32_t tmem_base;
 };
@@ -118,40 +134,46 @@ __device__ __forceinline__ void group_sync(int g) {
     asm volatile("bar.sync %0, %1;" ::"r"(g + 1), "n"(TC_GROUP_THREADS) : "memory");
 }
 
-// one 128 x 64 x 64 GEMM into TMEM columns [d_col, d_col + 64)
-template <int MODE>
+// one 128 x KW x KW GEMM into TMEM columns [d_col, d_col + KW)
+template <int MODE, int KW = 64>
 __device__ __forceinline__ void issue_gemm(uint32_t tmem_base, uint32_t d_col,
                                            const uint8_t *a_hi, const uint8_t *a_lo,
                                            const uint8_t *b_hi, const uint8_t *b_lo,
                                            uint64_t *bar) {
-    const uint64_t ah = make_desc(smem_u32(a_hi)), al = make_desc(smem_u32(a_lo));
-    const uint64_t bh = make_desc(smem_u32(b_hi)), bl = make_desc(smem_u32(b_lo));
     const uint32_t d = tmem_base + d_col;
-    constexpr uint32_t idesc = TcCfg<MODE>::F16 ? TC_IDESC_F16 : TC_IDESC;
+    constexpr uint32_t idesc = tc_idesc(KW, TcCfg<MODE, KW>::F16);
     uint32_t acc = 0;
 #pragma unroll
-    for (int ks = 0; ks < TC_K / 16; ++ks) {
-        const uint64_t adv = (uint64_t)(ks * 2);   // 16 elements = 32 B = 2 x 16 B
-        umma_bf16(d, ah + adv, bh + adv, idesc, acc);
-        acc = 1;
-        if (TcCfg<MODE>::A_LO) umma_bf16(d, al + adv, bh + adv, idesc, 1);
-        if (TcCfg<MODE>::B_LO) umma_bf16(d, ah + adv, bl + adv, idesc, 1);
+    for (int kb = 0; kb < KW / 64; ++kb) {
+        const uint64_t ah = make_desc(smem_u32(a_hi + kb * TE * 128));
+        const uint64_t al = make_desc(smem_u32(a_lo + kb * TE * 128));
+        const uint64_t bh = make_desc(smem_u32(b_hi + kb * KW * 128));
+        const uint64_t bl = make_desc(smem_u32(b_lo + kb * KW * 128));
+#pragma unroll
+        for (int ks = 0; ks < 4; ++ks) {
+            const uint64_t adv = (uint64_t)(ks * 2);   // 16 elements = 32 B = 2 x 16 B
+            umma_bf16(d, ah + adv, bh + adv, idesc, acc);
+            acc = 1;
+            if (TcCfg<MODE, KW>::A_LO) umma_bf16(d, al + adv, bh + adv, idesc, 1);
+            if (TcCfg<MODE, KW>::B_LO) umma_bf16(d, ah + adv, bl + adv, idesc, 1);
+        }
     }
     umma_commit(bar);
 }
 
-template <int MODE>
-__global__ void __launch_bounds__(TcCfg<MODE>::THREADS, 1)
+template <int MODE, int KW>
+__global__ void __launch_bounds__(TcCfg<MODE, KW>::THREADS, 1)
 egnn_edge_tc_kernel(const EdgeArgs a) {
     // SWIZZLE_128B tiles need 1024-byte alignment; the kernel has no static
     // shared memory, so the dynamic window starts at its (aligned) base.
     extern __shared__ __align__(1024) uint8_t smem_dyn[];
     pdl_launch_dependents();
-    constexpr int TC_GROUPS = TcCfg<MODE>::GROUPS, TC_THREADS = TcCfg<MODE>::THREADS;
-    constexpr bool X3 = TcCfg<MODE>::A_LO;            // hi + lo activation tiles
-    constexpr bool F16 = TcCfg<MODE>::F16;            // fp16 operands
-    constexpr bool EXACT = TcCfg<MODE>::EXACT_SILU;
-    TcSmem<MODE> &S = *reinterpret_cast<TcSmem<MODE> *>(smem_dyn);
+    constexpr int TC_GROUPS = TcCfg<MODE, KW>::GROUPS, TC_THREADS = TcCfg<MODE, KW>::THREADS;
+    constexpr bool X3 = TcCfg<MODE, KW>::A_LO;        // hi + lo activation tiles
+    constexpr bool F16 = TcCfg<MODE, KW>::F16;        // fp16 operands
+    constexpr bool EXACT = TcCfg<MODE, KW>::EXACT_SILU;
+    constexpr int KB = KW / 64, TC_K = KW;
+    TcSmem<MODE, KW> &S = *reinterpret_cast<TcSmem<MODE, KW> *>(smem_dyn);
     if ((smem_u32(smem_dyn) & 1023u) != 0u) __trap();
     const int g = threadIdx.x / TC_GROUP_THREADS;          // group
     const int tid = threadIdx.x % TC_GROUP_THREADS;        // thread in group
@@ -165,15 +187,33 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
     const bool f_eres = (a.flags & PVS_F_EDGE_RESIDUAL) && a.m_prev != nullptr;
 
     // ---- one-time setup (whole CTA) ----
-    if (F16) {
-        load_weight_tiles_f16(S.W2_hi, S.W2_lo, a.edge_w2, k, k, k);
-        load_weight_tiles_f16(S.Wc1_hi, S.Wc1_lo, a.coord_w1, k, k, k);
+    if constexpr (KW == 64) {
+        if (F16) {
+            load_weight_tiles_f16(S.W2_hi, S.W2_lo, a.edge_w2, k, k, k);
+            load_weight_tiles_f16(S.Wc1_hi, S.Wc1_lo, a.coord_w1, k, k, k);
+        } else {
+            load_weight_tiles<X3>(S.W2_hi, S.W2_lo, a.edge_w2, k, k, k);
+            load_weight_tiles<X3>(S.Wc1_hi, S.Wc1_lo, a.coord_w1, k, k, k);
+        }
     } else {
-        load_weight_tiles<X3>(S.W2_hi, S.W2_lo, a.edge_w2, k, k, k);
-        load_weight_tiles<X3>(S.Wc1_hi, S.Wc1_lo, a.coord_w1, k, k, k);
+        // K-block b: input channels [64 b, 64 b + 64) of all KW output rows
+        for (int b = 0; b < KB; ++b) {
+            const int o = b * KW * 128;
+            if (F16) {
+                load_weight_tiles_f16(S.W2_hi + o, S.W2_lo + o, a.edge_w2 + 64 * b, k, k,
+                                      k - 64 * b, KW);
+                load_weight_tiles_f16(S.Wc1_hi + o, S.Wc1_lo + o, a.coord_w1 + 64 * b, k, k,
+                                      k - 64 * b, KW);
+            } else {
+                load_weight_tiles<X3>(S.W2_hi + o, S.W2_lo + (X3 ? o : 0),
+                                      a.edge_w2 + 64 * b, k, k, k - 64 * b, KW);
+                load_weight_tiles<X3>(S.Wc1_hi + o, S.Wc1_lo + (X3 ? o : 0),
+                                      a.coord_w1 + 64 * b, k, k, k - 64 * b, KW);
+            }
+        }
     }
     const int col_r = (a.flags & PVS_F_PERM_INVARIANT) ? k : 2 * k;
-    for (int n = threadIdx.x; n < 64; n += TC_THREADS) {
+    for (int n = threadIdx.x; n < KW; n += TC_THREADS) {
         const bool ok = n < k;
         S.b2[n] = ok ? a.edge_b2[n] : 0.0f;
         S.bc1[n] = ok ? a.coord_b1[n] : 0.0f;
@@ -191,7 +231,7 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = S.tmem_base;
-    const uint32_t tmem_grp = tmem_base + (uint32_t)g * TC_GROUP_COLS;
+    const uint32_t tmem_grp = tmem_base + (uint32_t)g * (uint32_t)KW;
     const uint32_t tmem_lane = tmem_grp + ((uint32_t)(warp * 32) << 16);
     uint32_t phase = 0;
     const float att_b = (f_att && a.att_b) ? a.att_b[0] : 0.0f;
@@ -299,8 +339,10 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
                 // its last row; nobody reads what they produce) and run three
                 // passes ahead of the arithmetic, so a pass never waits for
                 // its own gather.
-                {
-                    const int c = tid & 7, slot = tid >> 3;
+                // (KW = 128: one sweep per 64-channel K-block)
+#pragma unroll 1
+                for (int kb = 0; kb < KB; ++kb) {
+                    const int c = (tid & 7) + 8 * kb, slot = tid >> 3;
                     float2 wr2[4];
 #pragma unroll
                     for (int i = 0; i < 4; ++i)
@@ -338,12 +380,12 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
                         silu4_mode<EXACT>(v[0], v[1]);
                         silu4_mode<EXACT>(v[2], v[3]);
                         if (F16) {
-                            *reinterpret_cast<uint4 *>(A_hi + swz(r, c)) = pack8_f16(v);
+                            *reinterpret_cast<uint4 *>(A_hi + swzk<KW>(r, c)) = pack8_f16(v);
                         } else {
                             uint4 hi, lo;
                             split8p<X3>(v, hi, lo);
-                            *reinterpret_cast<uint4 *>(A_hi + swz(r, c)) = hi;
-                            if (X3) *reinterpret_cast<uint4 *>(A_lo + swz(r, c)) = lo;
+                            *reinterpret_cast<uint4 *>(A_hi + swzk<KW>(r, c)) = hi;
+                            if (X3) *reinterpret_cast<uint4 *>(A_lo + swzk<KW>(r, c)) = lo;
                         }
                     };
 #pragma unroll
@@ -366,7 +408,7 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
                 // ---- GEMM 1: t2 = s1 . W2^T ----
                 if (tid == 0) {
                     tc_fence_after();
-                    issue_gemm<MODE>(tmem_grp, 0, A_hi, A_lo, S.W2_hi, S.W2_lo, &Gm.mbar);
+                    issue_gemm<MODE, KW>(tmem_grp, 0, A_hi, A_lo, S.W2_hi, S.W2_lo, &Gm.mbar);
                 }
                 mbar_wait(&Gm.mbar, phase);
                 phase ^= 1;
@@ -378,7 +420,7 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
                     const int r = tid;
                     float2 dot2 = make_float2(0.0f, 0.0f);
 #pragma unroll 1
-                    for (int q = 0; q < 4; ++q) {
+                    for (int q = 0; q < KW / 16; ++q) {
                         float acc[16];
                         tmem_ld16(tmem_lane + 16 * q, acc);
 #pragma unroll
@@ -421,12 +463,12 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
                             for (int i = 0; i < 4; ++i) dot2 = ffma2(wat[i], mv[i], dot2);
                             const int c = 2 * q + hlf;
                             if (F16) {
-                                *reinterpret_cast<uint4 *>(A_hi + swz(r, c)) = pack8_f16(mv);
+                                *reinterpret_cast<uint4 *>(A_hi + swzk<KW>(r, c)) = pack8_f16(mv);
                             } else {
                                 uint4 hi, lo;
                                 split8p<X3>(mv, hi, lo);
-                                *reinterpret_cast<uint4 *>(A_hi + swz(r, c)) = hi;
-                                if (X3) *reinterpret_cast<uint4 *>(A_lo + swz(r, c)) = lo;
+                                *reinterpret_cast<uint4 *>(A_hi + swzk<KW>(r, c)) = hi;
+                                if (X3) *reinterpret_cast<uint4 *>(A_lo + swzk<KW>(r, c)) = lo;
                             }
                         }
                     }
@@ -450,7 +492,7 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
                 // reduced below ----
                 if (f_coords && tid == 0) {
                     tc_fence_after();
-                    issue_gemm<MODE>(tmem_grp, 0, A_hi, A_lo, S.Wc1_hi, S.Wc1_lo, &Gm.mbar);
+                    issue_gemm<MODE, KW>(tmem_grp, 0, A_hi, A_lo, S.Wc1_hi, S.Wc1_lo, &Gm.mbar);
                 }
             }
             // ---- M_i = sum_e alpha_e m_e over dst segments: a warp per node,
@@ -458,14 +500,17 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
             // hi and of the lo tile each), partial sums folded by two shuffles.
             // The order of the additions is fixed, so the sums are reproducible.
             if (!f_softmax) {
-                const int es = lane >> 3, cc = lane & 7;
+                const int es = lane >> 3;
+#pragma unroll 1
+                for (int kb = 0; kb < KB; ++kb) {
+                const int cc = (lane & 7) + 8 * kb;
                 for (int nl = warp; nl < nn; nl += TC_GROUP_THREADS / 32) {
                     const int lo = Gm.rp[nl] - c0, hi = Gm.rp[nl + 1] - c0;
                     float2 s[4];
 #pragma unroll
                     for (int i = 0; i < 4; ++i) s[i] = make_float2(0.0f, 0.0f);
                     for (int el = lo + es; el < hi; el += 4) {
-                        const uint32_t off = swz(el, cc);
+                        const uint32_t off = swzk<KW>(el, cc);
                         const uint4 h = *reinterpret_cast<const uint4 *>(A_hi + off);
                         const float al = Gm.e_z[el];
                         const float2 al2 = make_float2(al, al);
@@ -503,12 +548,13 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
                         dst[1] = make_float4(s[2].x, s[2].y, s[3].x, s[3].y);
                     }
                 }
+                }   // K-blocks
             }
             // ---- messages out (edge residual of the next layer / softmax) ----
             if (a.m_out != nullptr) {
                 for (int idx = tid; idx < ne * (TC_K / 2); idx += TC_GROUP_THREADS) {
-                    const int el = idx >> 5, w = idx & 31;
-                    const uint32_t off = swz(el, w >> 2) + ((w & 3) << 2);
+                    const int el = idx / (TC_K / 2), w = idx % (TC_K / 2);
+                    const uint32_t off = swzk<KW>(el, w >> 2) + ((w & 3) << 2);
                     const uint32_t h = *reinterpret_cast<const uint32_t *>(A_hi + off);
                     float m0 = __uint_as_float(h << 16);
                     float m1 = __uint_as_float(h & 0xffff0000u);
@@ -536,7 +582,7 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
                 PHASE_MARK(5);
                 float2 d2 = make_float2(0.0f, 0.0f);
 #pragma unroll 1
-                for (int q = 0; q < 4; ++q) {
+                for (int q = 0; q < KW / 16; ++q) {
                     float acc[16];
                     tmem_ld16(tmem_lane + 16 * q, acc);
 #pragma unroll
@@ -610,8 +656,10 @@ egnn_edge_tc_kernel(const EdgeArgs a) {
 
 // Nodes cut by tile boundaries: the tile where such a node STARTS owns its
 // reduction and adds the partials of the following tiles in tile order.
+template <int KW>
 __global__ void __launch_bounds__(256)
 edge_tile_fixup_kernel(const EdgeArgs a, int do_m, int do_x) {
+    constexpr int TC_K = KW;
     pdl_launch_dependents();
     pdl_wait();
     const int t = blockIdx.x * 8 + (threadIdx.x >> 5), lane = threadIdx.x & 31;
@@ -623,21 +671,34 @@ edge_tile_fixup_kernel(const EdgeArgs a, int do_m, int do_x) {
     const int eb0 = a.row_ptr[b], eb1 = a.row_ptr[b + 1];
     if (eb1 <= E1) return;                         // the node ends in this tile
     if (eb0 < E0) return;                          // it started earlier: not the owner
-    float2 s = make_float2(0.f, 0.f);
+    // (KW = 128: a lane sums two channel pairs, 2 lane and 64 + 2 lane)
+    float2 s[KW / 64];
     float xs = 0.f;
-    if (do_m) s = *reinterpret_cast<const float2 *>(a.Mpart + ((size_t)t * 2 + 1) * TC_K + 2 * lane);
+#pragma unroll
+    for (int h = 0; h < KW / 64; ++h) {
+        s[h] = make_float2(0.f, 0.f);
+        if (do_m)
+            s[h] = *reinterpret_cast<const float2 *>(a.Mpart + ((size_t)t * 2 + 1) * TC_K + 64 * h +
+                                                     2 * lane);
+    }
     if (do_x && lane < 3) xs = a.xpart[((size_t)t * 2 + 1) * 4 + lane];
     for (int tt = t + 1; tt < n_tiles; ++tt) {
         if (do_m) {
-            const float2 p = *reinterpret_cast<const float2 *>(
-                a.Mpart + ((size_t)tt * 2) * TC_K + 2 * lane);
-            s.x += p.x;
-            s.y += p.y;
+#pragma unroll
+            for (int h = 0; h < KW / 64; ++h) {
+                const float2 p = *reinterpret_cast<const float2 *>(
+                    a.Mpart + ((size_t)tt * 2) * TC_K + 64 * h + 2 * lane);
+                s[h].x += p.x;
+                s[h].y += p.y;
+            }
         }
         if (do_x && lane < 3) xs += a.xpart[((size_t)tt * 2) * 4 + lane];
         if (eb1 <= min((tt + 1) * TE, E_total)) break;
     }
-    if (do_m) *reinterpret_cast<float2 *>(a.M + (size_t)b * TC_K + 2 * lane) = s;
+    if (do_m)
+#pragma unroll
+        for (int h = 0; h < KW / 64; ++h)
+            *reinterpret_cast<float2 *>(a.M + (size_t)b * TC_K + 64 * h + 2 * lane) = s[h];
     if (do_x && lane < 3)
         a.x_out[3 * b + lane] = a.x_in[3 * b + lane] + xs / (float)(eb1 - eb0);
 }
@@ -654,18 +715,20 @@ extern "C" int pvs_debug_phase_cycles(unsigned long long *out, int reset) {
 }
 #endif
 
-template <int MODE>
+template <int MODE, int KW = 64>
 static int launch_mode(const EdgeArgs &a, int n_ptiles_cap, cudaStream_t st) {
-    constexpr int G = TcCfg<MODE>::GROUPS;
-    const size_t smem = sizeof(TcSmem<MODE>);
+    constexpr int G = TcCfg<MODE, KW>::GROUPS;
+    static_assert(sizeof(TcSmem<MODE, KW>) <= 227 * 1024, "shared memory of one CTA");
+    static_assert(G * KW <= (int)TC_TMEM_COLS, "TMEM columns of one CTA");
+    const size_t smem = sizeof(TcSmem<MODE, KW>);
     int grid = num_sms();   // one persistent CTA per SM
     const int need = (n_ptiles_cap + G - 1) / G;
     if (need < grid) grid = need;
     if (grid < 1) grid = 1;
-    const int rc = ensure_smem(egnn_edge_tc_kernel<MODE>, smem);
+    const int rc = ensure_smem(egnn_edge_tc_kernel<MODE, KW>, smem);
     if (rc) return rc;
-    if (launch_chained(egnn_edge_tc_kernel<MODE>, dim3(grid), dim3(TcCfg<MODE>::THREADS), smem, st,
-                       a) != cudaSuccess)
+    if (launch_chained(egnn_edge_tc_kernel<MODE, KW>, dim3(grid), dim3(TcCfg<MODE, KW>::THREADS),
+                       smem, st, a) != cudaSuccess)
         return check_launch(0);
     return PVS_OK;
 }
@@ -680,16 +743,24 @@ int launch_edge_tc(const EdgeArgs &a, int n_ptiles_cap, int mode, cudaStream_t s
         const char *e = getenv("PVS_EDGE_TC8");
         return e ? atoi(e) : PVS_EDGE_TC8_DEFAULT;
     }();
-    if (mode == PVS_MATH_BF16X3 && tc8) rc = launch_edge_tc8(a, n_ptiles_cap, st);
+    // 65 <= k <= 128: the 128-wide tiles (forward only; P, Q, M at pitch 128)
+    const bool wide = a.k > 64;
+    if (wide && mode == PVS_MATH_BF16X3) rc = launch_mode<TCM_BF16X3, 128>(a, n_ptiles_cap, st);
+    else if (wide && mode == PVS_MATH_FP16X2) rc = launch_mode<TCM_FP16X2, 128>(a, n_ptiles_cap, st);
+    else if (wide) rc = launch_mode<TCM_BF16, 128>(a, n_ptiles_cap, st);
+    else if (mode == PVS_MATH_BF16X3 && tc8) rc = launch_edge_tc8(a, n_ptiles_cap, st);
     else if (mode == PVS_MATH_BF16X3) rc = launch_mode<TCM_BF16X3>(a, n_ptiles_cap, st);
     else if (mode == PVS_MATH_FP16X2) rc = launch_mode<TCM_FP16X2>(a, n_ptiles_cap, st);
     else rc = launch_mode<TCM_BF16>(a, n_ptiles_cap, st);
     if (rc) return rc;
     const bool softmax = (a.flags & PVS_F_EDGE_ATTENTION) && (a.flags & PVS_F_SOFTMAX_ATTENTION);
     const int do_m = softmax ? 0 : 1, do_x = a.x_out != nullptr ? 1 : 0;
-    if (do_m || do_x)
-        launch_chained(edge_tile_fixup_kernel, dim3((n_ptiles_cap + 7) / 8), dim3(256), 0, st, a,
-                       do_m, do_x);
+    if ((do_m || do_x) && wide)
+        launch_chained(edge_tile_fixup_kernel<128>, dim3((n_ptiles_cap + 7) / 8), dim3(256), 0,
+                       st, a, do_m, do_x);
+    else if (do_m || do_x)
+        launch_chained(edge_tile_fixup_kernel<64>, dim3((n_ptiles_cap + 7) / 8), dim3(256), 0, st,
+                       a, do_m, do_x);
     return check_launch(do_m || do_x ? 2 : 1);
 }
 

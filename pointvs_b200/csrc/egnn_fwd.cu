@@ -771,14 +771,15 @@ static FwdWorkspace carve_workspace(void *base, int n, int e, int kp, uint32_t f
     w.P = take((int64_t)n * kp);
     w.Q = take((int64_t)n * kp);
     w.M = take((int64_t)n * kp);
+    const int kv = kp > 64 ? kp : 64;   // channels of the per-channel vectors
     if (flags & PVS_F_GRAPHNORM) {
         w.V = take((int64_t)n * kp);
         w.gn_partial = take(GN_BLOCKS * 64);
-        w.gn_shift = take(64);
-        w.gn_a = take(64);
-        w.gn_b = take(64);
-        w.gn_mean = take(64);
-        w.gn_invstd = take(64);
+        w.gn_shift = take(kv);
+        w.gn_a = take(kv);
+        w.gn_b = take(kv);
+        w.gn_mean = take(kv);
+        w.gn_invstd = take(kv);
     }
     if ((flags & PVS_F_EDGE_ATTENTION) && (flags & PVS_F_SOFTMAX_ATTENTION)) {
         w.m_ws = take((int64_t)e * kp);
@@ -786,7 +787,7 @@ static FwdWorkspace carve_workspace(void *base, int n, int e, int kp, uint32_t f
     }
     {
         const int64_t tcap = pvs_packed_tiles_capacity(e);
-        w.Mpart = take(tcap * 2 * 64);
+        w.Mpart = take(tcap * 2 * kv);
         w.xpart = take(tcap * 2 * 4);
     }
     w.bytes = p - (char *)base;
@@ -795,17 +796,25 @@ static FwdWorkspace carve_workspace(void *base, int n, int e, int kp, uint32_t f
 
 // Batch-wide GraphNorm statistics of V (two passes: mean, then the centred
 // second moment) -> the per-channel affine gn_a * v + gn_b, mean and 1/std.
+// The kernels take 64 channels at a time: at pitch 128 (k > 64) the four
+// launches run once per 64-channel half, on offset pointers.
 static int graphnorm_stats(const FwdWorkspace &w, const pvs_layer_params *p, int n, int k,
                            int kp, cudaStream_t st) {
-    gn_colsum_kernel<<<GN_BLOCKS, 256, 0, st>>>(w.V, n, kp, nullptr, 0, w.gn_partial);
-    gn_finalize_kernel<<<1, 64, 0, st>>>(w.gn_partial, GN_BLOCKS, n, k, 0, p->gn_weight,
-                                         p->gn_bias, p->gn_mean_scale, w.gn_shift, w.gn_a,
-                                         w.gn_b, w.gn_mean, w.gn_invstd);
-    gn_colsum_kernel<<<GN_BLOCKS, 256, 0, st>>>(w.V, n, kp, w.gn_shift, 1, w.gn_partial);
-    gn_finalize_kernel<<<1, 64, 0, st>>>(w.gn_partial, GN_BLOCKS, n, k, 1, p->gn_weight,
-                                         p->gn_bias, p->gn_mean_scale, w.gn_shift, w.gn_a,
-                                         w.gn_b, w.gn_mean, w.gn_invstd);
-    return check_launch(4);
+    int launches = 0;
+    for (int c0 = 0; c0 < kp; c0 += 64) {
+        const int kc = k - c0;
+        const float *gw = p->gn_weight + c0, *gb = p->gn_bias + c0, *gm = p->gn_mean_scale + c0;
+        float *sh = w.gn_shift + c0, *ga = w.gn_a + c0, *gbo = w.gn_b + c0;
+        float *mean = w.gn_mean + c0, *inv = w.gn_invstd + c0;
+        gn_colsum_kernel<<<GN_BLOCKS, 256, 0, st>>>(w.V + c0, n, kp, nullptr, 0, w.gn_partial);
+        gn_finalize_kernel<<<1, 64, 0, st>>>(w.gn_partial, GN_BLOCKS, n, kc, 0, gw, gb, gm, sh, ga,
+                                             gbo, mean, inv);
+        gn_colsum_kernel<<<GN_BLOCKS, 256, 0, st>>>(w.V + c0, n, kp, sh, 1, w.gn_partial);
+        gn_finalize_kernel<<<1, 64, 0, st>>>(w.gn_partial, GN_BLOCKS, n, kc, 1, gw, gb, gm, sh, ga,
+                                             gbo, mean, inv);
+        launches += 4;
+    }
+    return check_launch(launches);
 }
 
 int64_t fwd_recompute_bytes(int n, int e, uint32_t flags) {
@@ -918,9 +927,10 @@ int pvs_mean_pool_fwd(const float *h, const int32_t *graph_ptr, int32_t n_graphs
 
 int64_t pvs_egnn_layer_workspace_bytes(int32_t n_nodes, int32_t n_edges,
                                        const pvs_layer_config *cfg) {
-    if (!cfg || cfg->k < 1 || cfg->k > PVS_MAX_K) return -1;
+    if (!cfg || cfg->k < 1 || cfg->k > PVS_MAX_K_TC_FWD) return -1;
     if (cfg->math < PVS_MATH_FP32 || cfg->math > PVS_MATH_FP16X2) return -1;
-    const int kp = (cfg->k <= 32 && cfg->math == PVS_MATH_FP32) ? 32 : 64;
+    if (cfg->k > PVS_MAX_K && cfg->math == PVS_MATH_FP32) return -1;
+    const int kp = cfg->k > 64 ? 128 : (cfg->k <= 32 && cfg->math == PVS_MATH_FP32) ? 32 : 64;
     return carve_workspace(nullptr, n_nodes, n_edges, kp, cfg->flags).bytes + 256;
 }
 
@@ -931,7 +941,9 @@ int pvs_egnn_layer_fwd(const pvs_graph *g, const pvs_layer_config *cfg,
                        float *natt_out, void *workspace, int64_t workspace_bytes,
                        void *stream) {
     if (!g || !cfg || !p) return PVS_ERR_INVALID_ARG;
-    if (cfg->k < 1 || cfg->k > PVS_MAX_K) return PVS_ERR_UNSUPPORTED_K;
+    // 65..128: forward only, on the tensor cores (the FFMA kernels are 64 wide)
+    if (cfg->k < 1 || cfg->k > PVS_MAX_K_TC_FWD) return PVS_ERR_UNSUPPORTED_K;
+    if (cfg->k > PVS_MAX_K && cfg->math == PVS_MATH_FP32) return PVS_ERR_UNSUPPORTED_K;
     if (cfg->math < PVS_MATH_FP32 || cfg->math > PVS_MATH_FP16X2) return PVS_ERR_INVALID_ARG;
     if (cfg->n_edge_classes < 0 || cfg->n_edge_classes > PVS_MAX_EDGE_CLASSES)
         return PVS_ERR_INVALID_ARG;
@@ -964,8 +976,8 @@ int pvs_egnn_layer_fwd(const pvs_graph *g, const pvs_layer_config *cfg,
 
     cudaStream_t st = (cudaStream_t)stream;
     const int k = cfg->k;
-    const bool tc = cfg->math != PVS_MATH_FP32;   // tcgen05 tiles are 64 wide
-    const int kp = (k <= 32 && !tc) ? 32 : 64;
+    const bool tc = cfg->math != PVS_MATH_FP32;   // tcgen05 tiles are 64 or 128 wide
+    const int kp = k > 64 ? 128 : (k <= 32 && !tc) ? 32 : 64;
     const int n = g->n_nodes, E = g->n_edges;
     const bool perm = f & PVS_F_PERM_INVARIANT;
     const int in_e = (perm ? k : 2 * k) + 1 + cfg->n_edge_classes;

@@ -59,12 +59,15 @@ ModelWs carve_model(void *base, int n, int e, int b, const pvs_model_desc *md) {
 
 int check_desc(const pvs_model_desc *md) {
     if (!md || md->n_layers < 0 || md->n_head < 1 || md->n_head > 3) return PVS_ERR_INVALID_ARG;
-    if (md->k < 1 || md->k > PVS_MAX_K) return PVS_ERR_UNSUPPORTED_K;
+    if (md->k < 1 || md->k > PVS_MAX_K_TC_FWD) return PVS_ERR_UNSUPPORTED_K;
     if (md->dim_input < 1 || md->dim_input > 128) return PVS_ERR_INVALID_ARG;
     if (!md->embed_w || !md->head || (md->n_layers > 0 && (!md->layer_cfg || !md->layer_params)))
         return PVS_ERR_INVALID_ARG;
-    for (int l = 0; l < md->n_layers; ++l)
+    for (int l = 0; l < md->n_layers; ++l) {
         if (md->layer_cfg[l].k != md->k) return PVS_ERR_INVALID_ARG;
+        if (md->k > PVS_MAX_K && md->layer_cfg[l].math == PVS_MATH_FP32)
+            return PVS_ERR_UNSUPPORTED_K;   // 65..128 runs on the tensor cores only
+    }
     for (int i = 0; i < md->n_head; ++i) {
         const pvs_head_layer &hl = md->head[i];
         if (!hl.w || hl.ki < 1 || hl.ki > 128 || hl.ko < 1 || hl.ko > 128) return PVS_ERR_INVALID_ARG;
@@ -181,6 +184,7 @@ int pvs_egnn_stack_fwd(const pvs_graph *g, int32_t n_layers, const pvs_layer_con
     const int n = g->n_nodes;
     if (n <= 0) return PVS_OK;
     const int k = cfgs[0].k;
+    if (k > PVS_MAX_K) return PVS_ERR_UNSUPPORTED_K;   // training path: 64 wide
     if (layer_ws_stride < stack_layer_ws_stride(n, g->n_edges, n_layers, cfgs))
         return PVS_ERR_WORKSPACE;
     cudaStream_t st = (cudaStream_t)stream;
@@ -213,6 +217,7 @@ int64_t pvs_egnn_stack_bwd_workspace_bytes(int32_t n_nodes, int32_t n_edges, int
     int64_t lw = 0;
     for (int l = 0; l < n_layers; ++l) {
         const int64_t v = pvs_egnn_layer_bwd_workspace_bytes(n_nodes, n_edges, &cfgs[l]);
+        if (v < 0) return -1;
         if (v > lw) lw = v;
     }
     const int k = cfgs[0].k;
@@ -232,6 +237,8 @@ int pvs_egnn_stack_bwd(const pvs_graph *g, const int32_t *csc_ptr, const int32_t
     if (!g || !cfgs || !params || !grads || !H || !X || !d_h_out || !d_h_in || !d_x_in ||
         !workspace || n_layers < 1)
         return PVS_ERR_INVALID_ARG;
+    for (int l = 0; l < n_layers; ++l)
+        if (cfgs[l].k < 1 || cfgs[l].k > PVS_MAX_K) return PVS_ERR_UNSUPPORTED_K;
     const int n = g->n_nodes;
     if (n <= 0) return PVS_OK;
     if (workspace_bytes < pvs_egnn_stack_bwd_workspace_bytes(n, g->n_edges, n_layers, cfgs))

@@ -1153,6 +1153,8 @@ int launch_node_bwd_tc(const NodeBwdArgs &a, cudaStream_t st) {
 int launch_node_pre_tc(const float *h, const float *edge_w1, const float *edge_b1, float *P,
                        float *Q, int n_nodes, int k, int in_e, int perm, int mode,
                        cudaStream_t st) {
+    if (k > 64)
+        return launch_wide_node_pre_tc(h, edge_w1, edge_b1, P, Q, n_nodes, k, in_e, perm, mode, st);
     NodePreArgs a{};
     a.h = h; a.edge_w1 = edge_w1; a.edge_b1 = edge_b1; a.P = P; a.Q = Q;
     a.n_nodes = n_nodes; a.k = k; a.in_e = in_e; a.perm_invariant = perm;
@@ -1187,6 +1189,9 @@ int launch_node_tc(const float *h_in, const float *M, float *h_out, float *natt_
                    const pvs_layer_params *p, int n_nodes, int k, uint32_t flags, int att_act,
                    int mode, cudaStream_t st, int phase, float *V, const float *gn_a,
                    const float *gn_b) {
+    if (k > 64)
+        return launch_wide_node_tc(h_in, M, h_out, natt_out, p, n_nodes, k, flags, att_act, mode,
+                                   st, phase, V, gn_a, gn_b);
     NodeTcArgs a{};
     a.phase = phase; a.V = V; a.gn_a = gn_a; a.gn_b = gn_b;
     a.h_in = h_in; a.M = M; a.h_out = h_out; a.natt_out = natt_out;

@@ -66,12 +66,22 @@ def _csr_for(edge_index, edge_attr, n_nodes):
 STAGE_TIMER = None
 
 
+def _width_error(k, fp32):
+    """Why the library refused hidden width k."""
+    if _cabi.MAX_K < k <= _cabi.MAX_K_TC_FWD and fp32:
+        return (f'hidden width k={k}: hidden width 65..128 needs a tensor-core '
+                "math mode (set_math('bf16x3'), 'fp16x2' or 'bf16')")
+    return (f'unsupported hidden width k={k} (1..{_cabi.MAX_K}; '
+            f'{_cabi.MAX_K + 1}..{_cabi.MAX_K_TC_FWD} for scoring in a '
+            'tensor-core math mode)')
+
+
 def _workspace(layer_cfg, n_nodes, n_edges, device):
     nbytes = int(lib().pvs_egnn_layer_workspace_bytes(
         n_nodes, n_edges, C.byref(layer_cfg)))
     if nbytes < 0:
-        raise _cabi.PvsError(
-            f'unsupported hidden width k={layer_cfg.k} (1..{_cabi.MAX_K})')
+        raise _cabi.PvsError(_width_error(
+            layer_cfg.k, layer_cfg.math == _cabi.MATH['fp32']))
     return torch.empty(nbytes, dtype=torch.uint8, device=device)
 
 
@@ -647,8 +657,9 @@ class PNNGeometricBase(PointNeuralNetworkBase):
             csr.n_nodes, csr.n_edges, n_graphs, C.byref(desc)))
         if nbytes < 0:
             raise _cabi.PvsError(
-                f'unsupported model for the fused scoring pass (k={desc.k}; '
-                f'hidden width must be 1..{_cabi.MAX_K})')
+                'unsupported model for the fused scoring pass: ' + _width_error(
+                    desc.k, any(cfgs[i].math == _cabi.MATH['fp32']
+                                for i in range(desc.n_layers))))
         ws = _cabi.scratch('model_fwd', nbytes, dev)
         scores = torch.empty((n_graphs, dim_out), dtype=torch.float32,
                              device=dev)

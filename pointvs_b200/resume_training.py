@@ -12,6 +12,7 @@ single `epochs` / `train_data_root` layout) and runs the remaining epochs:
 import argparse
 from pathlib import Path
 
+from .base import check_trainable_width
 from .data import get_data_loader
 from .load_model import load_model
 
@@ -54,6 +55,8 @@ def main(argv=None):
     parser.add_argument('--epochs_affinity', '-ea', type=int, default=-1)
     args = parser.parse_args(argv)
     base_path = Path(args.base_path).expanduser().resolve()
+    _, _, _, cmd = load_model(base_path, fetch_args_only=True)
+    check_trainable_width(cmd.get('channels', 0))
     _, model, _, cmd = load_model(base_path, init_path=True)
     ea, ep = args.epochs_affinity, args.epochs_pose
 

@@ -22,6 +22,7 @@ from pathlib import Path
 import torch
 import yaml
 
+from .base import check_trainable_width
 from .data import get_data_loader
 from .egnn import MultitaskSatorrasEGNN, SartorrasEGNN
 
@@ -142,6 +143,7 @@ def main(argv=None):
         raise NotImplementedError('--double: the CUDA path computes in fp32')
     if args.synth_pharm or args.synthpharm:
         raise NotImplementedError('synthpharm datasets are outside this path')
+    check_trainable_width(args.channels)
     if args.wandb_project is None:
         save_path = Path(args.save_path).expanduser()
     elif args.wandb_run is None:
