@@ -56,6 +56,7 @@ typedef enum pvs_status {
 #define PVS_CAP_FWD_FP16X2 8u    /* PVS_MATH_FP16X2 edge kernel               */
 #define PVS_CAP_CROP 16u         /* K0: pvs_crop_count / pvs_crop_fill        */
 #define PVS_CAP_FWD_WIDE_K 32u   /* forward at 65..PVS_MAX_K_TC_FWD (tcgen05)  */
+#define PVS_CAP_POCKET 64u       /* K1p: pvs_pocket_build_* / pvs_pocket_graph_* */
 
 /* pvs_layer_config.flags -- EGNNLayer.__init__ (egnn_satorras.py:26-46) */
 #define PVS_F_RESIDUAL 0x001u
@@ -265,6 +266,81 @@ int pvs_crop_fill(const double *lig_xyz, const uint8_t *lig_emit,
                   int32_t mask_words, const int32_t *complex_ptr,
                   int32_t n_atom_types, int32_t compact, double *coords,
                   int32_t *bp, float *feats, void *stream);
+
+/* ---- K1p: radius graph of ligand poses against resident receptors ----------
+ * Replaces: generate_edges (preprocessing/preprocessing.py:68-155) for the
+ *           complexes K0 assembles (data_loaders.py:259-309) when many poses
+ *           share a receptor.  The receptor-receptor part of every such graph
+ *           is the same, so it is searched once per pocket; per batch only
+ *           ligand-ligand and ligand-receptor pairs are tested.
+ * Output: exactly pvs_radius_graph_count / _fill's (deg, n_inter, row_ptr,
+ * col, attr, edge_capacity / overflow semantics) on the same K0 complexes,
+ * byte for byte: the same fp64 pair test, the same within-row order.
+ *
+ * A pocket is the receptors in K0's form (xyz fp64 [A][3], emit u8 [A],
+ * rec_ptr int32 [R+1]; they stay resident and K0 reads the same arrays)
+ * plus, in caller-allocated device memory:
+ *   cells  pvs_pocket_cells_bytes(R, A) bytes (about 128 KB per receptor
+ *          plus 28 B per atom): a cell list of each receptor's emitted
+ *          atoms (cell edge >= max radius, at most PVS_POCKET_MAX_DIM cells
+ *          per axis, larger cells beyond);
+ *   rr_ptr int32 [A+1], rr_col int32 [rr_ptr[A]]: CSR of the receptor-
+ *          receptor pairs within intra_radius over emitted atoms, rows in
+ *          concatenated atom order, columns the atom's index inside its own
+ *          receptor, ascending (file order).
+ * Build, once per pocket: pvs_pocket_build_count (cell list, rr_ptr; scratch
+ * pvs_pocket_build_scratch_bytes(R, A), free after the call), a host read
+ * of rr_ptr[A] to size rr_col, then pvs_pocket_build_fill.  A receptor of
+ * more than PVS_POCKET_MAX_REC_ATOMS atoms returns PVS_ERR_TOO_LARGE.
+ *
+ * Per batch, after K0 (pvs_crop_count / pvs_crop_fill):
+ *   coords, complex_ptr: K0's assembled complexes; mask / mask_words: K0's
+ *   keep bits (mask_words * 32 >= pocket->max_atoms); lig_count int32 [B]:
+ *   emitted ligand atoms of each pose, all <= max_ligand_atoms <=
+ *   PVS_POCKET_MAX_LIG_ATOMS (above: PVS_ERR_TOO_LARGE; a pose whose count
+ *   exceeds max_ligand_atoms gets no edges, and the fill sets *overflow to
+ *   2); rec_of_pose int32 [B] or NULL.
+ *   The radii must be the pocket's own (else PVS_ERR_INVALID_ARG).
+ *   scratch: pvs_scan_scratch_bytes(n_nodes). */
+#define PVS_POCKET_MAX_LIG_ATOMS 256    /* emitted ligand atoms per pose      */
+#define PVS_POCKET_MAX_REC_ATOMS 65536  /* atoms per receptor                 */
+#define PVS_POCKET_MAX_DIM 32           /* cells per axis of a receptor grid  */
+
+typedef struct pvs_pocket {
+    int32_t n_receptors;
+    int32_t n_atoms;        /* rec_ptr[n_receptors] */
+    int32_t max_atoms;      /* atoms of the largest receptor */
+    double inter_radius;    /* the radii the pocket is built for */
+    double intra_radius;
+    const double *xyz;      /* [n_atoms][3] */
+    const uint8_t *emit;    /* [n_atoms] */
+    const int32_t *rec_ptr; /* [n_receptors + 1] */
+    void *cells;            /* pvs_pocket_cells_bytes(n_receptors, n_atoms) */
+    int32_t *rr_ptr;        /* [n_atoms + 1] */
+    int32_t *rr_col;        /* [rr_ptr[n_atoms]] (build_fill and per batch) */
+} pvs_pocket;
+
+int64_t pvs_pocket_cells_bytes(int32_t n_receptors, int32_t n_atoms);
+int64_t pvs_pocket_build_scratch_bytes(int32_t n_receptors, int32_t n_atoms);
+int pvs_pocket_build_count(const pvs_pocket *pocket, void *scratch, void *stream);
+int pvs_pocket_build_fill(const pvs_pocket *pocket, void *stream);
+int pvs_pocket_graph_count(const pvs_pocket *pocket, const double *coords,
+                           const int32_t *complex_ptr, int32_t n_poses,
+                           int32_t n_nodes, const uint32_t *mask,
+                           int32_t mask_words, const int32_t *lig_count,
+                           int32_t max_ligand_atoms,
+                           const int32_t *rec_of_pose, double inter_radius,
+                           double intra_radius, int32_t *deg, int32_t *n_inter,
+                           int32_t *row_ptr, void *scratch, void *stream);
+int pvs_pocket_graph_fill(const pvs_pocket *pocket, const double *coords,
+                          const int32_t *complex_ptr, int32_t n_poses,
+                          int32_t n_nodes, const uint32_t *mask,
+                          int32_t mask_words, const int32_t *lig_count,
+                          int32_t max_ligand_atoms, const int32_t *rec_of_pose,
+                          double inter_radius, double intra_radius,
+                          int32_t *row_ptr, int32_t edge_capacity,
+                          int32_t *col, uint8_t *attr, int32_t *overflow,
+                          void *stream);
 
 int64_t pvs_scan_scratch_bytes(int32_t n);
 /* row_ptr[0..n] = exclusive scan of deg[0..n-1] */

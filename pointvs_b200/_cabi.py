@@ -37,6 +37,10 @@ CAP_FWD_FP32 = 1
 CAP_FWD_TCGEN05 = 2
 CAP_BWD_FP32 = 4
 CAP_FWD_WIDE_K = 32
+CAP_POCKET = 64
+
+POCKET_MAX_LIG_ATOMS = 256     # emitted ligand atoms per pose (K1p)
+POCKET_MAX_REC_ATOMS = 65536   # atoms per receptor of a pocket (K1p)
 
 _fp = C.c_void_p
 
@@ -86,6 +90,15 @@ class ModelDesc(C.Structure):
                 ('head', C.POINTER(HeadLayer))]
 
 
+class PocketDesc(C.Structure):
+    """struct pvs_pocket"""
+    _fields_ = [('n_receptors', C.c_int32), ('n_atoms', C.c_int32),
+                ('max_atoms', C.c_int32), ('inter_radius', C.c_double),
+                ('intra_radius', C.c_double), ('xyz', _fp), ('emit', _fp),
+                ('rec_ptr', _fp), ('cells', _fp), ('rr_ptr', _fp),
+                ('rr_col', _fp)]
+
+
 class PvsError(RuntimeError):
     pass
 
@@ -113,7 +126,9 @@ def lib():
                      'pvs_linear_bwd_workspace_bytes',
                      'pvs_egnn_layer_bwd_workspace_bytes',
                      'pvs_egnn_stack_layer_ws_stride',
-                     'pvs_egnn_stack_bwd_workspace_bytes'):
+                     'pvs_egnn_stack_bwd_workspace_bytes',
+                     'pvs_pocket_cells_bytes',
+                     'pvs_pocket_build_scratch_bytes'):
             if hasattr(handle, name):
                 getattr(handle, name).restype = C.c_int64
         _lib = handle

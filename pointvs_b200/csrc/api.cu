@@ -54,7 +54,7 @@ int pvs_version(void) { return PVS_VERSION; }
 
 uint32_t pvs_capabilities(void) {
     return PVS_CAP_FWD_FP32 | PVS_CAP_FWD_TCGEN05 | PVS_CAP_BWD_FP32 | PVS_CAP_FWD_FP16X2 |
-           PVS_CAP_CROP | PVS_CAP_FWD_WIDE_K;
+           PVS_CAP_CROP | PVS_CAP_FWD_WIDE_K | PVS_CAP_POCKET;
 }
 
 const char *pvs_status_string(int status) {
@@ -64,7 +64,8 @@ const char *pvs_status_string(int status) {
         case PVS_ERR_UNSUPPORTED_K:
             return "unsupported hidden width (1..64; 65..128 forward only, in a tensor-core "
                    "math mode)";
-        case PVS_ERR_TOO_LARGE: return "complex too large for the cell-list kernel";
+        case PVS_ERR_TOO_LARGE:
+            return "complex, receptor or ligand too large for the graph kernels";
         case PVS_ERR_CUDA: return "CUDA error (see pvs_last_cuda_error)";
         case PVS_ERR_WORKSPACE: return "workspace too small";
         case PVS_ERR_UNSUPPORTED: return "configuration not supported by the kernels yet";

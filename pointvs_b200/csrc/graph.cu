@@ -4,7 +4,7 @@
 //
 // Replaces /root/reference/point_vs/preprocessing/preprocessing.py:68-155
 // (generate_edges) and the PyG collate offsets (data_loaders.py:517-520).
-#include "pvs_common.cuh"
+#include "graph_common.cuh"
 
 namespace pvs {
 
@@ -14,27 +14,6 @@ namespace pvs {
 constexpr int SCAN_THREADS = 1024;
 constexpr int SCAN_ITEMS = 4;
 constexpr int SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
-
-// exclusive scan of one value per thread across the block; returns prefix,
-// writes the block total to *total (all threads see it after the call).
-__device__ int block_scan_excl(int v, int *total, int *warp_buf) {
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    const int nwarps = (blockDim.x + 31) >> 5;
-    int incl = warp_scan_incl(v, lane);
-    if (lane == 31) warp_buf[warp] = incl;
-    __syncthreads();
-    if (warp == 0) {
-        int w = lane < nwarps ? warp_buf[lane] : 0;
-        int wi = warp_scan_incl(w, lane);
-        warp_buf[lane] = wi - w;
-        if (lane == 31) warp_buf[32] = wi;
-    }
-    __syncthreads();
-    int prefix = warp_buf[warp] + incl - v;
-    *total = warp_buf[32];
-    __syncthreads();
-    return prefix;
-}
 
 __global__ void __launch_bounds__(SCAN_THREADS)
 scan_local_kernel(const int32_t *__restrict__ in, int n,
@@ -84,8 +63,8 @@ scan_add_kernel(int32_t *__restrict__ out, int n,
         if (base + i < n) out[base + i] += add;
 }
 
-static int exclusive_scan(const int32_t *deg, int n, int32_t *row_ptr,
-                          void *scratch, cudaStream_t st) {
+int exclusive_scan(const int32_t *deg, int n, int32_t *row_ptr, void *scratch,
+                   cudaStream_t st) {
     if (n == 0) {
         return cuda_call(cudaMemsetAsync(row_ptr, 0, sizeof(int32_t), st));
     }
@@ -95,24 +74,6 @@ static int exclusive_scan(const int32_t *deg, int n, int32_t *row_ptr,
     scan_sums_kernel<<<1, SCAN_THREADS, 0, st>>>(sums, nb, row_ptr + n);
     if (nb > 1) scan_add_kernel<<<nb, SCAN_THREADS, 0, st>>>(row_ptr, n, sums);
     return check_launch(nb > 1 ? 3 : 2);
-}
-
-// in-place exclusive scan of a shared-memory array of any length
-__device__ int smem_scan_excl(int *data, int n, int *warp_buf) {
-    const int T = blockDim.x;
-    const int per = (n + T - 1) / T;
-    const int lo = min(n, (int)threadIdx.x * per), hi = min(n, lo + per);
-    int s = 0;
-    for (int i = lo; i < hi; ++i) s += data[i];
-    int total;
-    int prefix = block_scan_excl(s, &total, warp_buf);
-    for (int i = lo; i < hi; ++i) {
-        int v = data[i];
-        data[i] = prefix;
-        prefix += v;
-    }
-    __syncthreads();
-    return total;
 }
 
 // ---------------------------------------------------------------------------
@@ -146,14 +107,6 @@ static size_t rg_smem_bytes(int max_n, bool with_prefix, bool stage) {
     b = (b + 7) & ~(size_t)7;
     if (stage) b += (size_t)max_n * (3 * sizeof(double) + sizeof(int));  // cell-sorted copy
     return b;
-}
-
-// cell index along one axis; `inv` = 1 / cell edge.  Monotone in v, and the same
-// expression bins the atoms and locates the query, so neighbours within r_max
-// (< cell edge / (1 + 1e-6)) are never more than one cell apart.
-__device__ __forceinline__ int cell_coord(double v, double lo, double inv, int dim) {
-    int c = (int)floor(__dmul_rn(__dsub_rn(v, lo), inv));
-    return max(0, min(dim - 1, c));
 }
 
 template <bool FILL>
@@ -283,11 +236,7 @@ radius_graph_kernel(const double *__restrict__ coords,
     __syncthreads();
 
     // ---- one warp per destination node ----
-    const double inter_lo = r_inter * r_inter * (1.0 - 1e-15);
-    const double inter_hi = r_inter * r_inter * (1.0 + 1e-15);
-    const double intra_lo = r_intra * r_intra * (1.0 - 1e-15);
-    const double intra_hi = r_intra * r_intra * (1.0 + 1e-15);
-    const double pos_hi = 1e-14 * (1.0 + 1e-15);
+    const PairBand band = pair_band(r_inter, r_intra);
     const int nw = (n + 31) / 32;
     // neighbour search of destination atom i by W lanes (lane index l):
     // sets the bits of its inter / intra neighbours in m_inter / m_intra
@@ -318,30 +267,9 @@ radius_graph_kernel(const double *__restrict__ coords,
                         xj = cx[3 * j]; yj = cx[3 * j + 1]; zj = cx[3 * j + 2];
                         bj = cbp[j];
                     }
-                    // scipy cdist (preprocessing.py:108):
-                    // sqrt((dx*dx + dy*dy) + dz*dz), no FMA contraction
-                    double ddx = __dsub_rn(xi, xj);
-                    double ddy = __dsub_rn(yi, yj);
-                    double ddz = __dsub_rn(zi, zj);
-                    const double d2 = __dadd_rn(
-                        __dadd_rn(__dmul_rn(ddx, ddx), __dmul_rn(ddy, ddy)),
-                        __dmul_rn(ddz, ddz));
-                    // The reference compares the ROUNDED sqrt with the radius.
-                    // Outside a +-1e-15 relative band around r^2 the outcome is
-                    // decided by d2 alone (sqrt is monotone and correctly
-                    // rounded); only inside the band is the sqrt evaluated.
+                    // scipy cdist (preprocessing.py:108), graph_common.cuh
                     bool pos, in_inter, in_intra;
-                    if (d2 > pos_hi && (d2 < inter_lo || d2 > inter_hi) &&
-                        (d2 < intra_lo || d2 > intra_hi)) {
-                        pos = true;
-                        in_inter = d2 < inter_lo;
-                        in_intra = d2 < intra_lo;
-                    } else {
-                        const double d = __dsqrt_rn(d2);
-                        pos = d > 1e-7;
-                        in_inter = d < r_inter;
-                        in_intra = d < r_intra;
-                    }
+                    pair_test(band, xi, yi, zi, xj, yj, zj, pos, in_inter, in_intra);
                     unsigned bit = 1u << (j & 31);
                     if (pos && in_inter && bj != bi)
                         atomicOr(&m_inter[j >> 5], bit);   // :110-117
@@ -409,26 +337,9 @@ radius_graph_kernel(const double *__restrict__ coords,
                             xj = cx[3 * j]; yj = cx[3 * j + 1]; zj = cx[3 * j + 2];
                             bj = cbp[j];
                         }
-                        // same arithmetic as `search` above (scipy cdist order,
-                        // no FMA contraction, sqrt only inside the 1e-15 band)
-                        const double ddx = __dsub_rn(xi, xj);
-                        const double ddy = __dsub_rn(yi, yj);
-                        const double ddz = __dsub_rn(zi, zj);
-                        const double d2 = __dadd_rn(
-                            __dadd_rn(__dmul_rn(ddx, ddx), __dmul_rn(ddy, ddy)),
-                            __dmul_rn(ddz, ddz));
+                        // the same test as `search` above
                         bool pos, in_inter, in_intra;
-                        if (d2 > pos_hi && (d2 < inter_lo || d2 > inter_hi) &&
-                            (d2 < intra_lo || d2 > intra_hi)) {
-                            pos = true;
-                            in_inter = d2 < inter_lo;
-                            in_intra = d2 < intra_lo;
-                        } else {
-                            const double d = __dsqrt_rn(d2);
-                            pos = d > 1e-7;
-                            in_inter = d < r_inter;
-                            in_intra = d < r_intra;
-                        }
+                        pair_test(band, xi, yi, zi, xj, yj, zj, pos, in_inter, in_intra);
                         const unsigned bit = 1u << (j & 31);
                         if (pos && in_inter && bj != bi) {       // :110-117
                             m_inter[j >> 5] |= bit;
@@ -896,6 +807,18 @@ __global__ void batch_to_ptr_kernel(const int64_t *__restrict__ batch, int n_nod
         if (g >= 0 && g <= n_graphs) ptr[g] = i;
 }
 
+// After a capacity-bounded fill: no consumer may index past col/attr, so the
+// offsets are cut at the capacity (a no-op unless *overflow was raised).
+__global__ void clamp_row_ptr_kernel(int32_t *row_ptr, int n, int cap) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n && row_ptr[i] > cap) row_ptr[i] = cap;
+}
+
+int clamp_row_ptr(int32_t *row_ptr, int n_nodes, int cap, cudaStream_t st) {
+    clamp_row_ptr_kernel<<<(n_nodes + 1 + 255) / 256, 256, 0, st>>>(row_ptr, n_nodes + 1, cap);
+    return check_launch();
+}
+
 }  // namespace pvs
 
 using namespace pvs;
@@ -999,18 +922,6 @@ __global__ void packed_tiles_kernel(const int32_t *__restrict__ row_ptr, int n_n
         if (row_ptr[mid] <= e) lo = mid; else hi = mid;
     }
     last[t] = lo;
-}
-
-// After a capacity-bounded fill: no consumer may index past col/attr, so the
-// offsets are cut at the capacity (a no-op unless *overflow was raised).
-__global__ void clamp_row_ptr_kernel(int32_t *row_ptr, int n, int cap) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    if (i < n && row_ptr[i] > cap) row_ptr[i] = cap;
-}
-
-static int clamp_row_ptr(int32_t *row_ptr, int n_nodes, int cap, cudaStream_t st) {
-    clamp_row_ptr_kernel<<<(n_nodes + 1 + 255) / 256, 256, 0, st>>>(row_ptr, n_nodes + 1, cap);
-    return check_launch();
 }
 
 int pvs_radius_graph_fill(const double *coords, const int32_t *bp,

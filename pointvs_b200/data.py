@@ -293,6 +293,29 @@ def crop_batch(ligands, receptors, rec_of_pose, radius, n_features, compact,
     receptor tensors must already be complete on the device (synchronise once
     after uploading them), or pass receptors_pending=True to order the side
     stream after the caller's stream."""
+    out = crop_batch_masked(ligands, receptors, rec_of_pose, radius, n_features,
+                            compact, device, receptors_pending)
+    return out.coords, out.bp, out.feats, out.complex_ptr_host
+
+
+class CropOutput:
+    """What K0 leaves on the device for one batch: the assembled complexes,
+    their offsets (host and device), and the per-pose receptor keep bits
+    (`mask_words` uint32 words per pose) that K1p consumes."""
+    __slots__ = ('coords', 'bp', 'feats', 'complex_ptr_host', 'complex_ptr',
+                 'mask', 'mask_words', 'rec_of_pose')
+
+    def __init__(self, **kw):
+        for k, v in kw.items():
+            setattr(self, k, v)
+
+
+def crop_batch_masked(ligands, receptors, rec_of_pose, radius, n_features,
+                      compact, device, receptors_pending=False,
+                      concatenated=None):
+    """`crop_batch` that also returns K0's keep-bit mask (-> CropOutput).
+    concatenated: the receptors already concatenated, (xyz, emit, code), so
+    a resident pocket skips the per-batch copy."""
     import ctypes as C   # noqa: PLC0415
     from . import _cabi   # noqa: PLC0415
     from ._cabi import check, lib, ptr, stream   # noqa: PLC0415
@@ -300,10 +323,13 @@ def crop_batch(ligands, receptors, rec_of_pose, radius, n_features, compact,
     n_poses = len(ligands)
     feature_dim = n_features + 1 if compact else 2 * n_features
     if n_poses == 0:
-        return (torch.zeros((0, 3), dtype=torch.float64, device=device),
-                torch.zeros(0, dtype=torch.int32, device=device),
-                torch.zeros((0, feature_dim), device=device),
-                np.zeros(1, dtype=np.int32))
+        return CropOutput(
+            coords=torch.zeros((0, 3), dtype=torch.float64, device=device),
+            bp=torch.zeros(0, dtype=torch.int32, device=device),
+            feats=torch.zeros((0, feature_dim), device=device),
+            complex_ptr_host=np.zeros(1, dtype=np.int32),
+            complex_ptr=torch.zeros(1, dtype=torch.int32, device=device),
+            mask=None, mask_words=0, rec_of_pose=None)
     rec_sizes = [int(r[0].shape[0]) for r in receptors]
     rec_ptr = np.zeros(len(receptors) + 1, dtype=np.int32)
     np.cumsum(rec_sizes, out=rec_ptr[1:])
@@ -320,7 +346,9 @@ def crop_batch(ligands, receptors, rec_of_pose, radius, n_features, compact,
     if receptors_pending:
         side.wait_stream(main)
     with torch.cuda.device(device), torch.cuda.stream(side):
-        if len(receptors) == 1:
+        if concatenated is not None:
+            rec_xyz, rec_emit, rec_code = concatenated
+        elif len(receptors) == 1:
             rec_xyz, rec_emit, rec_code = receptors[0]
         else:
             rec_xyz = torch.cat([r[0] for r in receptors])
@@ -367,7 +395,9 @@ def crop_batch(ligands, receptors, rec_of_pose, radius, n_features, compact,
         for t in (lig_xyz, lig_emit, lig_code, lig_ptr_d, rec_ptr_d,
                   rec_of_pose_d, mask, cptr, rec_xyz, rec_code):
             t.record_stream(main)
-    return coords[:n], bp[:n], feats[:n], cptr_host
+    return CropOutput(coords=coords[:n], bp=bp[:n], feats=feats[:n],
+                      complex_ptr_host=cptr_host, complex_ptr=cptr, mask=mask,
+                      mask_words=words, rec_of_pose=rec_of_pose_d)
 
 
 # --------------------------------------------------------------------------
@@ -820,5 +850,5 @@ def get_data_loader(data_root, dataset_class=None, receptors=None,
 __all__ = ['ComplexDataset', 'PackedLoader', 'get_data_loader',
            'parse_classification_types', 'parse_regression_types',
            'read_structure', 'build_complex', 'make_box', 'make_bit_vector',
-           'atomic_number_table', 'atom_codes', 'crop_batch', 'Complex',
-           'Ligand']
+           'atomic_number_table', 'atom_codes', 'crop_batch',
+           'crop_batch_masked', 'CropOutput', 'Complex', 'Ligand']
