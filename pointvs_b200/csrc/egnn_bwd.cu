@@ -1348,17 +1348,10 @@ int pvs_egnn_layer_bwd(const pvs_graph *g, const int32_t *csc_ptr, const int32_t
     cudaStream_t st = (cudaStream_t)stream;
     const BwdSide *side = g_bwd_side;
     // the backward kernels of a layer form a launch chain (pvs_common.cuh)
-    struct ChainScope {
-        bool prev;
-        ChainScope() : prev(g_pdl_chain) {
-            static const bool off = getenv("PVS_NO_PDL") != nullptr;
-            g_pdl_chain = !off;
-        }
-        ~ChainScope() { g_pdl_chain = prev; }
-    } chain_scope;
+    ChainScope chain_scope;
     const int k = cfg->k, n = g->n_nodes, E = g->n_edges;
     const bool perm = f & PVS_F_PERM_INVARIANT;
-    const int in_e = (perm ? k : 2 * k) + 1 + cfg->n_edge_classes;
+    const int in_e = edge_in_width(cfg);
     const int col_r = perm ? k : 2 * k;
     BwdWorkspace w = carve_bwd((void *)align_up((int64_t)(uintptr_t)workspace, 256), n, E, f);
     int rc;
@@ -1368,7 +1361,7 @@ int pvs_egnn_layer_bwd(const pvs_graph *g, const int32_t *csc_ptr, const int32_t
     FwdWorkspace fw{};
     if (cfg->saved_fwd_workspace != nullptr && cfg->math != PVS_MATH_FP32 && !softmax &&
         !graphnorm) {
-        fw = fwd_saved(cfg->saved_fwd_workspace, n, E, f);
+        fw = fwd_saved(cfg->saved_fwd_workspace, n, E, cfg);
     } else {
         rc = fwd_recompute(g, cfg, p, h_in, x_in, m_prev, w.fwd, &fw, st);
         if (rc) return rc;

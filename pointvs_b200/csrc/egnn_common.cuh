@@ -33,14 +33,18 @@ struct EdgeArgs {
     int att_act;
 };
 
+// columns of edge_mlp.0.weight: h_i and h_j (perm-invariant: h_i alone), the
+// squared distance and the one-hot edge class
+inline int edge_in_width(const pvs_layer_config *cfg) {
+    const int k = cfg->k;
+    return ((cfg->flags & PVS_F_PERM_INVARIANT) ? k : 2 * k) + 1 + cfg->n_edge_classes;
+}
 
 // launches the tcgen05 edge kernel (egnn_edge_tc.cu); mode = pvs_math
 int launch_edge_tc(const EdgeArgs &a, int n_ptiles_cap, int mode, cudaStream_t st);
 // bf16x3 variant with 8-warp groups and the segment-reduce on the tensor core
 // (egnn_edge_tc8.cu); launch_edge_tc dispatches to it when PVS_EDGE_TC8 says so
 int launch_edge_tc8(const EdgeArgs &a, int n_ptiles_cap, cudaStream_t st);
-// FFMA edge kernel with the 64-wide internal pitch (egnn_fwd.cu)
-int launch_edge_fp32_k64(const EdgeArgs &a, int n_tiles_cap, cudaStream_t st);
 // out = act(in . W^T + b) (w_in_major: out = in . W); accumulate: out += ...
 int launch_linear(const float *in, int ld_in, int rows, int ki, const float *w,
                   int ld_w, const float *b, int ko, int act, float *out,
@@ -53,6 +57,7 @@ struct FwdWorkspace {
     float *P, *Q, *M, *V, *m_ws, *z_ws, *gn_partial, *gn_shift, *gn_a, *gn_b;
     float *gn_mean, *gn_invstd;
     float *Mpart, *xpart;    // split-node partials of the edge-packed tiles
+    int kp;                  // pitch of P, Q, M, V and m_ws
     int64_t bytes;
 };
 int64_t fwd_recompute_bytes(int n, int e, uint32_t flags);
@@ -60,7 +65,7 @@ int fwd_recompute(const pvs_graph *g, const pvs_layer_config *cfg, const pvs_lay
                   const float *h_in, const float *x_in, const float *m_prev, void *ws_base,
                   FwdWorkspace *out, cudaStream_t st);
 // P, Q, M of a layer as pvs_egnn_layer_fwd left them in its workspace
-FwdWorkspace fwd_saved(const void *saved_workspace, int n, int e, uint32_t flags);
+FwdWorkspace fwd_saved(const void *saved_workspace, int n, int e, const pvs_layer_config *cfg);
 // tensor-core node stages (egnn_node_tc.cu); mode = PVS_MATH_BF16X3 / BF16
 // K3: d_h[N][k] += dP[N][64] . W1a + dQ[N][64] . W1b on tcgen05 (bf16x3)
 int launch_dgrad_pq_tc(const float *dP, const float *dQ, const float *edge_w1, float *d_h,

@@ -742,10 +742,6 @@ static int launch_edge(const EdgeArgs &a, int n_tiles_cap, cudaStream_t st) {
     return check_launch();
 }
 
-int launch_edge_fp32_k64(const EdgeArgs &a, int n_tiles_cap, cudaStream_t st) {
-    return launch_edge<64>(a, n_tiles_cap, st);
-}
-
 template <int KP>
 static int launch_node(const NodeArgs &a, cudaStream_t st) {
     size_t smem = ((size_t)3 * KP * 64 + (size_t)NODE_ROWS * (2 * KP + 4) +
@@ -760,9 +756,22 @@ static int launch_node(const NodeArgs &a, cudaStream_t st) {
 
 constexpr int GN_BLOCKS = 128;
 
-static FwdWorkspace carve_workspace(void *base, int n, int e, int kp, uint32_t flags) {
+// Pitch of P, Q, M and V in pvs_egnn_layer_fwd's workspace: the tcgen05 tiles
+// are 64 or 128 wide, the FFMA kernels 32 or 64.
+static int layer_pitch(const pvs_layer_config *cfg) {
+    return cfg->k > 64 ? 128 : (cfg->k <= 32 && cfg->math == PVS_MATH_FP32) ? 32 : 64;
+}
+// The backward kernels read P, Q, M and V at pitch 64: its recompute writes
+// them at that pitch whatever the forward's, and it reads the forward's own
+// workspace (fwd_saved) only where layer_pitch is 64 too.
+constexpr int RECOMPUTE_PITCH = 64;
+
+// The one layout of a layer's forward workspace, from `base` rounded up to 256 B.
+static FwdWorkspace carve_workspace(const void *base, int n, int e, int kp, uint32_t flags) {
     FwdWorkspace w{};
-    char *p = (char *)base;
+    w.kp = kp;
+    char *const start = (char *)align_up((int64_t)(uintptr_t)base, 256);
+    char *p = start;
     auto take = [&](int64_t count) {
         float *r = (float *)p;
         p += align_up(count * (int64_t)sizeof(float), 256);
@@ -790,7 +799,7 @@ static FwdWorkspace carve_workspace(void *base, int n, int e, int kp, uint32_t f
         w.Mpart = take(tcap * 2 * kv);
         w.xpart = take(tcap * 2 * 4);
     }
-    w.bytes = p - (char *)base;
+    w.bytes = p - start;
     return w;
 }
 
@@ -799,7 +808,8 @@ static FwdWorkspace carve_workspace(void *base, int n, int e, int kp, uint32_t f
 // The kernels take 64 channels at a time: at pitch 128 (k > 64) the four
 // launches run once per 64-channel half, on offset pointers.
 static int graphnorm_stats(const FwdWorkspace &w, const pvs_layer_params *p, int n, int k,
-                           int kp, cudaStream_t st) {
+                           cudaStream_t st) {
+    const int kp = w.kp;
     int launches = 0;
     for (int c0 = 0; c0 < kp; c0 += 64) {
         const int kc = k - c0;
@@ -818,84 +828,149 @@ static int graphnorm_stats(const FwdWorkspace &w, const pvs_layer_params *p, int
 }
 
 int64_t fwd_recompute_bytes(int n, int e, uint32_t flags) {
-    return carve_workspace(nullptr, n, e, 64, flags).bytes + 256;
+    return carve_workspace(nullptr, n, e, RECOMPUTE_PITCH, flags).bytes + 256;
 }
 
-// Forward recompute for the backward pass (64-wide pitch): P, Q, M (and the
-// softmax attention values + messages, and the GraphNorm pre-activation V with
-// its batch statistics).  No h_out / x_out is produced.
-FwdWorkspace fwd_saved(const void *saved_workspace, int n, int e, uint32_t flags) {
-    // same carve as pvs_egnn_layer_fwd in the tensor-core modes (pitch 64)
-    return carve_workspace((void *)align_up((int64_t)(uintptr_t)saved_workspace, 256), n, e, 64,
-                           flags);
+FwdWorkspace fwd_saved(const void *saved_workspace, int n, int e, const pvs_layer_config *cfg) {
+    return carve_workspace(saved_workspace, n, e, layer_pitch(cfg), cfg->flags);
 }
 
-int fwd_recompute(const pvs_graph *g, const pvs_layer_config *cfg, const pvs_layer_params *p,
-                  const float *h_in, const float *x_in, const float *m_prev, void *ws_base,
-                  FwdWorkspace *out, cudaStream_t st) {
-    const uint32_t f = cfg->flags;
-    const int k = cfg->k, n = g->n_nodes, E = g->n_edges;
-    const bool tc = cfg->math != PVS_MATH_FP32;
-    const bool perm = f & PVS_F_PERM_INVARIANT;
-    const int in_e = (perm ? k : 2 * k) + 1 + cfg->n_edge_classes;
-    const bool softmax = (f & PVS_F_EDGE_ATTENTION) && (f & PVS_F_SOFTMAX_ATTENTION);
-    FwdWorkspace w = carve_workspace((void *)align_up((int64_t)(uintptr_t)ws_base, 256), n, E, 64, f);
+// node_pre: P = h W1a^T + b1 ; Q = h W1b^T (perm-invariant: Q = h W1a^T)
+static int node_pre_stage(const pvs_layer_config *cfg, const pvs_layer_params *p,
+                          const float *h_in, int n, const FwdWorkspace &w, cudaStream_t st) {
+    const int k = cfg->k, in_e = edge_in_width(cfg);
+    const bool perm = cfg->flags & PVS_F_PERM_INVARIANT;
+    if (cfg->math != PVS_MATH_FP32)
+        return launch_node_pre_tc(h_in, p->edge_w1, p->edge_b1, w.P, w.Q, n, k, in_e,
+                                  perm ? 1 : 0, cfg->math, st);
     int rc;
-    if (tc) {
-        rc = launch_node_pre_tc(h_in, p->edge_w1, p->edge_b1, w.P, w.Q, n, k, in_e, perm ? 1 : 0,
-                                cfg->math, st);
-        if (rc) return rc;
-    } else {
-        if (k < 64) {
-            rc = cuda_call(cudaMemsetAsync(w.P, 0, (size_t)((char *)w.M - (char *)w.P), st));
-            if (rc) return rc;
-        }
-        rc = launch_linear(h_in, k, n, k, p->edge_w1, in_e, p->edge_b1, k, PVS_ACT_NONE, w.P, 64, st);
-        if (rc) return rc;
-        rc = launch_linear(h_in, k, n, k, p->edge_w1 + (perm ? 0 : k), in_e, nullptr, k,
-                           PVS_ACT_NONE, w.Q, 64, st);
+    if (k < w.kp) {
+        rc = cuda_call(cudaMemsetAsync(w.P, 0, (size_t)((char *)w.M - (char *)w.P), st));
         if (rc) return rc;
     }
+    rc = launch_linear(h_in, k, n, k, p->edge_w1, in_e, p->edge_b1, k, PVS_ACT_NONE, w.P, w.kp,
+                       st);
+    if (rc) return rc;
+    return launch_linear(h_in, k, n, k, p->edge_w1 + (perm ? 0 : k), in_e, nullptr, k,
+                         PVS_ACT_NONE, w.Q, w.kp, st);
+}
+
+// edge: messages, their sums M and the coordinate update; with softmax
+// attention, the aggregation over each node's segment.  edge_events records
+// cfg->ev_edge_begin / ev_edge_end around the stage.
+static int edge_stage(const pvs_graph *g, const pvs_layer_config *cfg, const pvs_layer_params *p,
+                      const float *x_in, const float *m_prev, float *x_out, float *m_out,
+                      float *att_out, const FwdWorkspace &w, bool edge_events, cudaStream_t st) {
+    const uint32_t f = cfg->flags;
+    const int n = g->n_nodes;
+    const bool softmax = (f & PVS_F_EDGE_ATTENTION) && (f & PVS_F_SOFTMAX_ATTENTION);
     EdgeArgs ea{};
     ea.row_ptr = g->row_ptr; ea.col = g->col; ea.tile_ptr = g->tile_ptr;
     ea.n_tiles = g->n_tiles; ea.attr = cfg->n_edge_classes > 0 ? g->attr : nullptr;
     ea.ptile_last = g->ptile_last; ea.n_ptiles = g->n_ptiles; ea.n_nodes = n;
     ea.Mpart = w.Mpart; ea.xpart = w.xpart;
     ea.P = w.P; ea.Q = w.Q; ea.x_in = x_in; ea.m_prev = m_prev; ea.M = w.M;
-    ea.x_out = nullptr;
-    ea.m_out = softmax ? w.m_ws : nullptr; ea.ld_m = 64;
-    ea.att_out = softmax ? w.z_ws : nullptr;
+    ea.x_out = x_out;
+    // the softmax pass needs every message and logit of a segment
+    ea.m_out = m_out ? m_out : softmax ? w.m_ws : nullptr;
+    ea.ld_m = m_out ? cfg->k : w.kp;
+    ea.att_out = att_out ? att_out : softmax ? w.z_ws : nullptr;
     ea.edge_w1 = p->edge_w1; ea.edge_w2 = p->edge_w2; ea.edge_b2 = p->edge_b2;
     ea.coord_w1 = p->coord_w1 ? p->coord_w1 : p->edge_w2;
     ea.coord_b1 = p->coord_b1 ? p->coord_b1 : p->edge_b2;
     ea.coord_w2 = p->coord_w2 ? p->coord_w2 : p->edge_b2;
     ea.att_w = p->att_w; ea.att_b = p->att_b; ea.edge_gate = p->edge_gate;
-    ea.k = k; ea.in_e = in_e; ea.n_classes = cfg->n_edge_classes;
+    ea.k = cfg->k; ea.in_e = edge_in_width(cfg); ea.n_classes = cfg->n_edge_classes;
     ea.flags = f; ea.att_act = cfg->att_act;
-    rc = tc ? launch_edge_tc(ea, g->n_ptiles_cap, cfg->math, st)
-            : launch_edge<64>(ea, g->n_tiles_cap, st);
+    if (edge_events && cfg->ev_edge_begin) cudaEventRecord((cudaEvent_t)cfg->ev_edge_begin, st);
+    int rc;
+    if (cfg->math != PVS_MATH_FP32) rc = launch_edge_tc(ea, g->n_ptiles_cap, cfg->math, st);
+    else rc = w.kp == 32 ? launch_edge<32>(ea, g->n_tiles_cap, st)
+                         : launch_edge<64>(ea, g->n_tiles_cap, st);
     if (rc) return rc;
     if (softmax) {
-        segment_softmax_agg_kernel<<<(n + 7) / 8, 256, 0, st>>>(g->row_ptr, n, w.m_ws, 64, 64,
-                                                               w.z_ws, w.M);
+        segment_softmax_agg_kernel<<<(n + 7) / 8, 256, 0, st>>>(
+            g->row_ptr, n, ea.m_out, ea.ld_m, w.kp, ea.att_out, w.M);
         rc = check_launch();
         if (rc) return rc;
     }
-    if (f & PVS_F_GRAPHNORM) {
-        NodeArgs na{};
-        na.h_in = h_in; na.M = w.M; na.h_out = nullptr; na.V = w.V;
-        na.node_w1 = p->node_w1; na.node_b1 = p->node_b1; na.node_w2 = p->node_w2;
-        na.node_b2 = p->node_b2; na.natt_w = p->natt_w; na.natt_b = p->natt_b;
-        na.node_gate = p->node_gate;
-        na.n_nodes = n; na.k = k; na.flags = f; na.att_act = cfg->att_act;
-        na.phase = 1;
-        rc = tc ? launch_node_tc(h_in, w.M, nullptr, nullptr, p, n, k, f, cfg->att_act,
-                                 cfg->math, st, 1, w.V, nullptr, nullptr)
-                : launch_node<64>(na, st);
-        if (rc) return rc;
-        rc = graphnorm_stats(w, p, n, k, 64, st);
+    if (edge_events && cfg->ev_edge_end) cudaEventRecord((cudaEvent_t)cfg->ev_edge_end, st);
+    return PVS_OK;
+}
+
+// FULL: the node model, h_out and natt_out.  GN_STATS: only GraphNorm's
+// pre-activation V and its batch statistics (nothing without GraphNorm).
+enum class NodeStage { FULL, GN_STATS };
+
+// node: phase 0, or with GraphNorm phase 1 (Wn1 -> V), the batch statistics
+// and phase 2 (resume from V)
+static int node_stage(const pvs_layer_config *cfg, const pvs_layer_params *p, const float *h_in,
+                      float *h_out, float *natt_out, int n, const FwdWorkspace &w,
+                      NodeStage mode, cudaStream_t st) {
+    const uint32_t f = cfg->flags;
+    const int k = cfg->k;
+    const bool graphnorm = f & PVS_F_GRAPHNORM;
+    if (mode == NodeStage::GN_STATS && !graphnorm) return PVS_OK;
+    NodeArgs na{};   // the FFMA kernel's
+    na.h_in = h_in; na.M = w.M; na.h_out = h_out; na.V = w.V;
+    na.natt_out = natt_out;
+    na.node_w1 = p->node_w1; na.node_b1 = p->node_b1; na.node_w2 = p->node_w2;
+    na.node_b2 = p->node_b2; na.natt_w = p->natt_w; na.natt_b = p->natt_b;
+    na.node_gate = p->node_gate;
+    na.n_nodes = n; na.k = k; na.flags = f; na.att_act = cfg->att_act;
+    auto run = [&](int phase) {
+        if (cfg->math != PVS_MATH_FP32) {
+            const bool out = phase != 1;
+            return launch_node_tc(h_in, w.M, out ? h_out : nullptr, out ? natt_out : nullptr, p,
+                                  n, k, f, cfg->att_act, cfg->math, st, phase,
+                                  phase ? w.V : nullptr, phase == 2 ? w.gn_a : nullptr,
+                                  phase == 2 ? w.gn_b : nullptr);
+        }
+        na.phase = phase;
+        if (phase == 2) { na.gn_a = w.gn_a; na.gn_b = w.gn_b; }
+        return w.kp == 32 ? launch_node<32>(na, st) : launch_node<64>(na, st);
+    };
+    if (!graphnorm) return run(0);
+    int rc = run(1);
+    if (rc) return rc;
+    rc = graphnorm_stats(w, p, n, k, st);
+    if (rc || mode == NodeStage::GN_STATS) return rc;
+    return run(2);
+}
+
+// One layer forward, over the stages set in `stages` (node_pre -> edge ->
+// node), on the workspace w.  Each output may be null.
+static int layer_forward(const pvs_graph *g, const pvs_layer_config *cfg,
+                         const pvs_layer_params *p, const float *h_in, const float *x_in,
+                         const float *m_prev, float *h_out, float *x_out, float *m_out,
+                         float *att_out, float *natt_out, const FwdWorkspace &w, int stages,
+                         bool edge_events, NodeStage node, cudaStream_t st) {
+    int rc;
+    if (stages & PVS_STAGE_NODE_PRE) {
+        rc = node_pre_stage(cfg, p, h_in, g->n_nodes, w, st);
         if (rc) return rc;
     }
+    if (stages & PVS_STAGE_EDGE) {
+        rc = edge_stage(g, cfg, p, x_in, m_prev, x_out, m_out, att_out, w, edge_events, st);
+        if (rc) return rc;
+    }
+    if (!(stages & PVS_STAGE_NODE)) return PVS_OK;
+    return node_stage(cfg, p, h_in, h_out, natt_out, g->n_nodes, w, node, st);
+}
+
+// Forward recompute for the backward pass: P, Q, M (and the softmax attention
+// values + messages, and the GraphNorm pre-activation V with its batch
+// statistics).  No h_out / x_out is produced; cfg->stages and the edge events
+// do not apply.
+int fwd_recompute(const pvs_graph *g, const pvs_layer_config *cfg, const pvs_layer_params *p,
+                  const float *h_in, const float *x_in, const float *m_prev, void *ws_base,
+                  FwdWorkspace *out, cudaStream_t st) {
+    const FwdWorkspace w =
+        carve_workspace(ws_base, g->n_nodes, g->n_edges, RECOMPUTE_PITCH, cfg->flags);
+    const int rc = layer_forward(g, cfg, p, h_in, x_in, m_prev, nullptr, nullptr, nullptr,
+                                 nullptr, nullptr, w, PVS_STAGE_ALL, false, NodeStage::GN_STATS,
+                                 st);
+    if (rc) return rc;
     *out = w;
     return PVS_OK;
 }
@@ -930,8 +1005,7 @@ int64_t pvs_egnn_layer_workspace_bytes(int32_t n_nodes, int32_t n_edges,
     if (!cfg || cfg->k < 1 || cfg->k > PVS_MAX_K_TC_FWD) return -1;
     if (cfg->math < PVS_MATH_FP32 || cfg->math > PVS_MATH_FP16X2) return -1;
     if (cfg->k > PVS_MAX_K && cfg->math == PVS_MATH_FP32) return -1;
-    const int kp = cfg->k > 64 ? 128 : (cfg->k <= 32 && cfg->math == PVS_MATH_FP32) ? 32 : 64;
-    return carve_workspace(nullptr, n_nodes, n_edges, kp, cfg->flags).bytes + 256;
+    return carve_workspace(nullptr, n_nodes, n_edges, layer_pitch(cfg), cfg->flags).bytes + 256;
 }
 
 int pvs_egnn_layer_fwd(const pvs_graph *g, const pvs_layer_config *cfg,
@@ -974,108 +1048,12 @@ int pvs_egnn_layer_fwd(const pvs_graph *g, const pvs_layer_config *cfg,
     if (workspace_bytes < pvs_egnn_layer_workspace_bytes(g->n_nodes, g->n_edges, cfg))
         return PVS_ERR_WORKSPACE;
 
-    cudaStream_t st = (cudaStream_t)stream;
-    const int k = cfg->k;
-    const bool tc = cfg->math != PVS_MATH_FP32;   // tcgen05 tiles are 64 or 128 wide
-    const int kp = k > 64 ? 128 : (k <= 32 && !tc) ? 32 : 64;
-    const int n = g->n_nodes, E = g->n_edges;
-    const bool perm = f & PVS_F_PERM_INVARIANT;
-    const int in_e = (perm ? k : 2 * k) + 1 + cfg->n_edge_classes;
-    void *ws_base = (void *)align_up((int64_t)(uintptr_t)workspace, 256);
-    FwdWorkspace w = carve_workspace(ws_base, n, E, kp, f);
-    const bool softmax = (f & PVS_F_EDGE_ATTENTION) && (f & PVS_F_SOFTMAX_ATTENTION);
-    int rc;
-
     const int stages = (cfg->stages & PVS_STAGE_ALL) ? (cfg->stages & PVS_STAGE_ALL)
                                                      : PVS_STAGE_ALL;
-    // node_pre: P = h W1a^T + b1 ; Q = h W1b^T (perm-invariant: Q = h W1a^T)
-    const bool tc_node = tc;
-    if ((stages & PVS_STAGE_NODE_PRE) && tc_node) {
-        rc = launch_node_pre_tc(h_in, p->edge_w1, p->edge_b1, w.P, w.Q, n, k, in_e, perm ? 1 : 0,
-                                cfg->math, st);
-        if (rc) return rc;
-    } else if (stages & PVS_STAGE_NODE_PRE) {
-    if (k < kp) {
-        rc = cuda_call(cudaMemsetAsync(w.P, 0, (size_t)((char *)w.M - (char *)w.P), st));
-        if (rc) return rc;
-    }
-    rc = launch_linear(h_in, k, n, k, p->edge_w1, in_e, p->edge_b1, k, PVS_ACT_NONE,
-                       w.P, kp, st);
-    if (rc) return rc;
-    rc = launch_linear(h_in, k, n, k, p->edge_w1 + (perm ? 0 : k), in_e, nullptr, k,
-                       PVS_ACT_NONE, w.Q, kp, st);
-    if (rc) return rc;
-    }
-
-    EdgeArgs ea{};
-    ea.row_ptr = g->row_ptr; ea.col = g->col; ea.tile_ptr = g->tile_ptr;
-    ea.n_tiles = g->n_tiles; ea.attr = cfg->n_edge_classes > 0 ? g->attr : nullptr;
-    ea.ptile_last = g->ptile_last; ea.n_ptiles = g->n_ptiles; ea.n_nodes = n;
-    ea.Mpart = w.Mpart; ea.xpart = w.xpart;
-    ea.P = w.P; ea.Q = w.Q; ea.x_in = x_in; ea.m_prev = m_prev; ea.M = w.M;
-    ea.x_out = x_out;
-    ea.m_out = m_out; ea.ld_m = k;
-    ea.att_out = att_out;
-    if (softmax) {
-        // the softmax pass needs every message and logit of a segment
-        if (m_out == nullptr) { ea.m_out = w.m_ws; ea.ld_m = kp; }
-        if (att_out == nullptr) ea.att_out = w.z_ws;
-    }
-    ea.edge_w1 = p->edge_w1; ea.edge_w2 = p->edge_w2; ea.edge_b2 = p->edge_b2;
-    ea.coord_w1 = p->coord_w1 ? p->coord_w1 : p->edge_w2;
-    ea.coord_b1 = p->coord_b1 ? p->coord_b1 : p->edge_b2;
-    ea.coord_w2 = p->coord_w2 ? p->coord_w2 : p->edge_b2;
-    ea.att_w = p->att_w; ea.att_b = p->att_b; ea.edge_gate = p->edge_gate;
-    ea.k = k; ea.in_e = in_e; ea.n_classes = cfg->n_edge_classes;
-    ea.flags = f; ea.att_act = cfg->att_act;
-    if (stages & PVS_STAGE_EDGE) {
-    if (cfg->ev_edge_begin) cudaEventRecord((cudaEvent_t)cfg->ev_edge_begin, st);
-    if (tc) rc = launch_edge_tc(ea, g->n_ptiles_cap, cfg->math, st);
-    else rc = kp == 32 ? launch_edge<32>(ea, g->n_tiles_cap, st)
-                       : launch_edge<64>(ea, g->n_tiles_cap, st);
-    if (rc) return rc;
-    }
-    if (softmax && (stages & PVS_STAGE_EDGE)) {
-        segment_softmax_agg_kernel<<<(n + 7) / 8, 256, 0, st>>>(
-            g->row_ptr, n, ea.m_out, ea.ld_m, kp, ea.att_out, w.M);
-        rc = check_launch();
-        if (rc) return rc;
-    }
-    if ((stages & PVS_STAGE_EDGE) && cfg->ev_edge_end)
-        cudaEventRecord((cudaEvent_t)cfg->ev_edge_end, st);
-
-    if (!(stages & PVS_STAGE_NODE)) return PVS_OK;
-    if (tc_node && !(f & PVS_F_GRAPHNORM))
-        return launch_node_tc(h_in, w.M, h_out, natt_out, p, n, k, f, cfg->att_act, cfg->math, st);
-    if (tc_node) {
-        // GraphNorm: Wn1 on the tensor cores -> V, batch statistics, resume from V
-        rc = launch_node_tc(h_in, w.M, nullptr, nullptr, p, n, k, f, cfg->att_act, cfg->math, st,
-                            1, w.V, nullptr, nullptr);
-        if (rc) return rc;
-        rc = graphnorm_stats(w, p, n, k, kp, st);
-        if (rc) return rc;
-        return launch_node_tc(h_in, w.M, h_out, natt_out, p, n, k, f, cfg->att_act, cfg->math, st,
-                              2, w.V, w.gn_a, w.gn_b);
-    }
-    NodeArgs na{};
-    na.h_in = h_in; na.M = w.M; na.h_out = h_out; na.V = w.V;
-    na.natt_out = natt_out;
-    na.node_w1 = p->node_w1; na.node_b1 = p->node_b1; na.node_w2 = p->node_w2;
-    na.node_b2 = p->node_b2; na.natt_w = p->natt_w; na.natt_b = p->natt_b;
-    na.node_gate = p->node_gate;
-    na.n_nodes = n; na.k = k; na.flags = f; na.att_act = cfg->att_act;
-    if (f & PVS_F_GRAPHNORM) {
-        na.phase = 1;
-        rc = kp == 32 ? launch_node<32>(na, st) : launch_node<64>(na, st);
-        if (rc) return rc;
-        rc = graphnorm_stats(w, p, n, k, kp, st);
-        if (rc) return rc;
-        na.phase = 2;
-        na.gn_a = w.gn_a; na.gn_b = w.gn_b;
-    } else {
-        na.phase = 0;
-    }
-    return kp == 32 ? launch_node<32>(na, st) : launch_node<64>(na, st);
+    const FwdWorkspace w =
+        carve_workspace(workspace, g->n_nodes, g->n_edges, layer_pitch(cfg), f);
+    return layer_forward(g, cfg, p, h_in, x_in, m_prev, h_out, x_out, m_out, att_out, natt_out,
+                         w, stages, true, NodeStage::FULL, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -17,14 +17,6 @@ struct ModelWs {
     int64_t bytes;
 };
 
-struct ChainScope {
-    ChainScope() {
-        static const bool off = getenv("PVS_NO_PDL") != nullptr;   // A/B switch
-        g_pdl_chain = !off;
-    }
-    ~ChainScope() { g_pdl_chain = false; }
-};
-
 bool any_edge_residual(const pvs_model_desc *md) {
     for (int l = 0; l < md->n_layers; ++l)
         if (md->layer_cfg[l].flags & PVS_F_EDGE_RESIDUAL) return true;

@@ -4,6 +4,7 @@
 #include <stdint.h>
 
 #include <atomic>
+#include <cstdlib>
 
 #include "pvs_b200.h"
 
@@ -45,8 +46,20 @@ __device__ __forceinline__ void pdl_launch_dependents() {
 __device__ __forceinline__ void pdl_wait() {
     asm volatile("griddepcontrol.wait;" ::: "memory");
 }
-// true while pvs_egnn_model_fwd / pvs_egnn_stack_fwd issue their layer chain
+// true while pvs_egnn_model_fwd / pvs_egnn_stack_fwd / pvs_egnn_layer_bwd issue
+// their launch chain
 extern thread_local bool g_pdl_chain;
+
+// Chains the launches of its lifetime (unless PVS_NO_PDL is set, the A/B
+// switch) and restores the previous setting on exit.
+struct ChainScope {
+    bool prev;
+    ChainScope() : prev(g_pdl_chain) {
+        static const bool off = getenv("PVS_NO_PDL") != nullptr;
+        g_pdl_chain = !off;
+    }
+    ~ChainScope() { g_pdl_chain = prev; }
+};
 
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_chained(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem,
