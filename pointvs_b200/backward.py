@@ -94,8 +94,11 @@ def egnn_layer_backward(ctx, d_h, d_x, d_m):
     layer, csr = ctx.layer, ctx.csr
     h, x, m_prev, *params = ctx.saved_tensors
     cfg = layer.c_config()
+    # differentiate the function the forward evaluated, also when set_math()
+    # ran in between
+    cfg.math = _cabi.MATH[ctx.fwd_math]
     fwd_ws = getattr(ctx, 'fwd_ws', None)
-    if fwd_ws is not None and getattr(ctx, 'fwd_math', None) == layer.math:
+    if fwd_ws is not None:
         cfg.saved_fwd_workspace = ptr(fwd_ws)
     n, e, k = csr.n_nodes, csr.n_edges, layer.hidden_nf
     dev = h.device
@@ -219,6 +222,7 @@ def egnn_stack_backward(ctx, d_h, d_x):
     span_params = []
     for i, layer in enumerate(layers):
         cfgs[i] = layer.c_config()
+        cfgs[i].math = _cabi.MATH[ctx.math]     # the forward's, as in the layer
         ps = params[i * per:(i + 1) * per]
         det = [None if p is None else p.detach().contiguous() for p in ps]
         keep.append(det)
@@ -243,12 +247,11 @@ def egnn_stack_backward(ctx, d_h, d_x):
     d_x_in = torch.empty_like(X[0])
     nbytes = int(lib().pvs_egnn_stack_bwd_workspace_bytes(n, e, L, cfgs))
     bws = torch.empty(nbytes, dtype=torch.uint8, device=dev)
-    use_saved = ctx.math == layers[0].math
     g = csr.c_struct()
     with torch.cuda.device(dev):
         check(lib().pvs_egnn_stack_bwd(
             C.byref(g), ptr(csc_ptr), ptr(csc_eid), L, cfgs, pstructs, gstructs,
-            ptr(H), ptr(X), ptr(ws) if use_saved else None,
+            ptr(H), ptr(X), ptr(ws),
             C.c_int64(ctx.stride), ptr(d_h), ptr(d_x), ptr(d_h_in), ptr(d_x_in),
             ptr(bws), C.c_int64(bws.numel()), stream()), 'pvs_egnn_stack_bwd')
     if arena is not None and arena.reduce_in_backward and span_params:
