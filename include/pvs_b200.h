@@ -301,7 +301,16 @@ int pvs_crop_fill(const double *lig_xyz, const uint8_t *lig_emit,
  *   exceeds max_ligand_atoms gets no edges, and the fill sets *overflow to
  *   2); rec_of_pose int32 [B] or NULL.
  *   The radii must be the pocket's own (else PVS_ERR_INVALID_ARG).
- *   scratch: pvs_scan_scratch_bytes(n_nodes). */
+ *   scratch: pvs_scan_scratch_bytes(n_nodes) (no more: the receptor rows of
+ *   a pose walk only its kept atoms, located from the keep bits in shared
+ *   memory, on as many CTAs as its kept count needs).
+ *
+ * Compose: pvs_pocket_compose fills `out`, a pocket of the receptors of
+ * parts[0], parts[1], ... in that order, from those built pockets by device
+ * copies, without searching any receptor again.  The caller gives `out` its
+ * concatenated xyz / emit / rec_ptr, sizes (n_receptors, n_atoms, max_atoms:
+ * the sums and the largest), the parts' radii, and cells, rr_ptr and rr_col
+ * sized for it (rr_col: the sum of the parts' rr_ptr[n_atoms]). */
 #define PVS_POCKET_MAX_LIG_ATOMS 256    /* emitted ligand atoms per pose      */
 #define PVS_POCKET_MAX_REC_ATOMS 65536  /* atoms per receptor                 */
 #define PVS_POCKET_MAX_DIM 32           /* cells per axis of a receptor grid  */
@@ -324,6 +333,8 @@ int64_t pvs_pocket_cells_bytes(int32_t n_receptors, int32_t n_atoms);
 int64_t pvs_pocket_build_scratch_bytes(int32_t n_receptors, int32_t n_atoms);
 int pvs_pocket_build_count(const pvs_pocket *pocket, void *scratch, void *stream);
 int pvs_pocket_build_fill(const pvs_pocket *pocket, void *stream);
+int pvs_pocket_compose(const pvs_pocket *const *parts, int32_t n_parts,
+                       const pvs_pocket *out, void *stream);
 int pvs_pocket_graph_count(const pvs_pocket *pocket, const double *coords,
                            const int32_t *complex_ptr, int32_t n_poses,
                            int32_t n_nodes, const uint32_t *mask,

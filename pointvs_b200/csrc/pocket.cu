@@ -257,6 +257,28 @@ pocket_rr_kernel(const double *__restrict__ xyz, const uint8_t *__restrict__ emi
 // ---------------------------------------------------------------------------
 // per batch: gridDim.y = `split` CTAs per pose
 // ---------------------------------------------------------------------------
+// CTAs of a pose's receptor rows: one per PG_ATOMS_PER_CTA kept atoms, at
+// least one, at most PG_MAX_SPLIT
+__host__ __device__ __forceinline__ int pg_split_of(int atoms) {
+    const int s = (atoms + PG_ATOMS_PER_CTA - 1) / PG_ATOMS_PER_CTA;
+    return s < 1 ? 1 : (s > PG_MAX_SPLIT ? PG_MAX_SPLIT : s);
+}
+
+// position of the set bit of rank k (0-based) in m; k < __popc(m)
+__device__ __forceinline__ int nth_set_bit(uint32_t m, int k) {
+    int p = 0;
+#pragma unroll
+    for (int s = 16; s > 0; s >>= 1) {
+        const int c = __popc(m & ((1u << s) - 1u));
+        if (k >= c) {
+            k -= c;
+            m >>= s;
+            p += s;
+        }
+    }
+    return p;
+}
+
 static size_t pg_smem_bytes(int max_lig, int mask_words) {
     return (size_t)(3 * max_lig + 6) * sizeof(double) +
            (size_t)(2 + 2 * PG_WARPS) * mask_words * sizeof(uint32_t) + 33 * sizeof(int);
@@ -310,7 +332,8 @@ pocket_graph_kernel(PocketCells c, const double *__restrict__ rec_xyz,
     }
     const uint32_t *mrow = mask + (size_t)b * mask_words;
     for (int w = tid; w < words; w += PG_THREADS) {
-        const uint32_t v = mrow[w];
+        // no bit at or above nr: kept atom t always lands on an atom j < nr
+        const uint32_t v = mrow[w] & (nr - 32 * w >= 32 ? ~0u : (1u << (nr - 32 * w)) - 1u);
         mw[w] = v;
         wp[w] = __popc(v);
     }
@@ -338,7 +361,7 @@ pocket_graph_kernel(PocketCells c, const double *__restrict__ rec_xyz,
             }
         }
     }
-    smem_scan_excl(wp, words, warp_buf);   // its barriers also publish lbox
+    const int kept_total = smem_scan_excl(wp, words, warp_buf);   // its barriers also publish lbox
 
     auto kept = [&](int j) { return (mw[j >> 5] >> (j & 31)) & 1u; };
     auto node = [&](int j) {   // complex-local node of kept receptor atom j
@@ -353,13 +376,25 @@ pocket_graph_kernel(PocketCells c, const double *__restrict__ rec_xyz,
         }
     };
 
-    // ---- receptor rows: a thread per receptor atom of this CTA's slice ----
+    // ---- receptor rows: a thread per kept receptor atom of this CTA's slice ----
     auto receptor_rows = [&]() {
-        const int j_lo = (int)(((long long)nr * part) / split);
-        const int j_hi = (int)(((long long)nr * (part + 1)) / split);
-        for (int j = j_lo + tid; j < j_hi; j += PG_THREADS) {
-            if (!kept(j)) continue;
-            const int row = n0 + node(j);
+        // the pose's kept atoms t = 0 .. n - nl - 1 are nodes nl + t; the pose
+        // uses as many of the grid's CTAs as its kept count needs
+        const int n_kept = min(n - nl, kept_total);
+        const int used = pg_split_of(n_kept);
+        if (part >= used) return;
+        const int t_lo = (int)(((long long)n_kept * part) / used);
+        const int t_hi = (int)(((long long)n_kept * (part + 1)) / used);
+        for (int t = t_lo + tid; t < t_hi; t += PG_THREADS) {
+            // kept atom t: the last word with wp[w] <= t, then the bit of rank
+            // t - wp[w] inside it
+            int w_lo = 0, w_hi = words;   // wp[w_lo] <= t < wp[w_hi], wp[words] = kept_total
+            while (w_hi - w_lo > 1) {
+                const int mid = (w_lo + w_hi) >> 1;
+                if (wp[mid] <= t) w_lo = mid; else w_hi = mid;
+            }
+            const int j = w_lo * 32 + nth_set_bit(mw[w_lo], t - wp[w_lo]);
+            const int row = n0 + nl + t;
             const double xj = rec_xyz[3 * (size_t)(r0 + j)], yj = rec_xyz[3 * (size_t)(r0 + j) + 1],
                          zj = rec_xyz[3 * (size_t)(r0 + j) + 2];
             const bool near = nl > 0 && xj > lbox[0] && xj < lbox[3] && yj > lbox[1] &&
@@ -484,6 +519,39 @@ pocket_graph_kernel(PocketCells c, const double *__restrict__ rec_xyz,
         receptor_rows();
 }
 
+// ---------------------------------------------------------------------------
+// compose: part k of a pocket of several receptors, copied from a built
+// pocket.  Cell positions are relative to rec_ptr[r] and rr_col holds indices
+// inside the receptor, so only rr_ptr moves: by the edges of the parts before
+// (out.rr_ptr[a_off], written by part k - 1's launch; 0 for the first part).
+// ---------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+pocket_compose_kernel(PocketCells src, const int32_t *__restrict__ src_rr_ptr,
+                      const int32_t *__restrict__ src_rr_col, int n_rec, int n_atoms,
+                      PocketCells dst, int32_t *__restrict__ dst_rr_ptr,
+                      int32_t *__restrict__ dst_rr_col, int r_off, int a_off, bool first) {
+    const int64_t i0 = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    const int64_t step = (int64_t)gridDim.x * blockDim.x;
+    const int32_t e_off = first ? 0 : dst_rr_ptr[a_off];
+    for (int64_t i = i0; i < 6 * n_rec; i += step) dst.geom[6 * (int64_t)r_off + i] = src.geom[i];
+    for (int64_t i = i0; i < 4 * n_rec; i += step) dst.dims[4 * (int64_t)r_off + i] = src.dims[i];
+    const int64_t n_cs = (int64_t)n_rec * (PK_MAX_CELLS + 1);
+    for (int64_t i = i0; i < n_cs; i += step)
+        dst.cell_start[(int64_t)r_off * (PK_MAX_CELLS + 1) + i] = src.cell_start[i];
+    for (int64_t i = i0; i < n_atoms; i += step) {
+        dst.cell_atom[a_off + i] = src.cell_atom[i];
+        dst.cell_xyz[3 * (a_off + i)] = src.cell_xyz[3 * i];
+        dst.cell_xyz[3 * (a_off + i) + 1] = src.cell_xyz[3 * i + 1];
+        dst.cell_xyz[3 * (a_off + i) + 2] = src.cell_xyz[3 * i + 2];
+    }
+    // entry a_off is the previous part's end (or 0): write 1 .. n_atoms
+    if (first && i0 == 0) dst_rr_ptr[0] = 0;
+    for (int64_t i = i0 + 1; i <= n_atoms; i += step)
+        dst_rr_ptr[a_off + i] = src_rr_ptr[i] + e_off;
+    const int32_t n_e = src_rr_ptr[n_atoms];
+    for (int64_t e = i0; e < n_e; e += step) dst_rr_col[e_off + e] = src_rr_col[e];
+}
+
 }  // namespace pvs
 
 using namespace pvs;
@@ -521,11 +589,6 @@ static int pose_check(const pvs_pocket *p, const double *coords, const int32_t *
     return PVS_OK;
 }
 
-static int pg_split(const pvs_pocket *p) {
-    int s = (p->max_atoms + PG_ATOMS_PER_CTA - 1) / PG_ATOMS_PER_CTA;
-    return s < 1 ? 1 : (s > PG_MAX_SPLIT ? PG_MAX_SPLIT : s);
-}
-
 template <bool FILL>
 static int pg_launch(const pvs_pocket *p, const double *coords, const int32_t *complex_ptr,
                      int32_t n_poses, const uint32_t *mask, int32_t mask_words,
@@ -541,9 +604,11 @@ static int pg_launch(const pvs_pocket *p, const double *coords, const int32_t *c
     if (rc) return rc;
     PocketCells c;
     cells_layout(p->cells, p->n_receptors, p->n_atoms, &c);
-    // receptor rows: CTAs by receptor size; ligand rows: no more CTAs than
-    // the largest ligand has warps' worth of atoms
-    const dim3 grid(n_poses, pg_split(p));
+    // receptor rows: enough CTAs for a pose that keeps the largest receptor
+    // whole; each pose runs on pg_split_of(its kept count) of them and the
+    // rest return at once.  Ligand rows: no more CTAs than the largest ligand
+    // has warps' worth of atoms
+    const dim3 grid(n_poses, pg_split_of(p->max_atoms));
     const int ml = max_lig > 0 ? max_lig : 1;
     const dim3 grid_lig(n_poses, std::min<int>(grid.y, (ml + PG_WARPS - 1) / PG_WARPS));
     const PairBand band = pair_band(r_inter, r_intra);
@@ -612,6 +677,50 @@ int pvs_pocket_build_fill(const pvs_pocket *pocket, void *stream) {
         p.xyz, p.emit, p.rec_ptr, pair_band(p.inter_radius, p.intra_radius), c, p.rr_ptr,
         p.rr_col);
     return check_launch();
+}
+
+int pvs_pocket_compose(const pvs_pocket *const *parts, int32_t n_parts, const pvs_pocket *out,
+                       void *stream) {
+    int rc = pocket_check(out);
+    if (rc) return rc;
+    if (n_parts < 1 || !parts) return PVS_ERR_INVALID_ARG;
+    int64_t n_rec = 0, n_atoms = 0;
+    int max_atoms = 0;
+    for (int k = 0; k < n_parts; ++k) {
+        const pvs_pocket *q = parts[k];
+        rc = pocket_check(q);
+        if (rc) return rc;
+        if (q->inter_radius != out->inter_radius || q->intra_radius != out->intra_radius)
+            return PVS_ERR_INVALID_ARG;
+        if (q->n_atoms > 0 && (!q->rr_col || !q->cells)) return PVS_ERR_INVALID_ARG;
+        n_rec += q->n_receptors;
+        n_atoms += q->n_atoms;
+        max_atoms = std::max(max_atoms, (int)q->max_atoms);
+    }
+    if (n_rec != out->n_receptors || n_atoms != out->n_atoms || max_atoms != out->max_atoms)
+        return PVS_ERR_INVALID_ARG;
+    if (!out->rr_ptr || (out->n_atoms > 0 && (!out->rr_col || !out->cells)))
+        return PVS_ERR_INVALID_ARG;
+    if (!out->cells) return out->n_receptors > 0 ? PVS_ERR_INVALID_ARG : PVS_OK;
+    PocketCells dst;
+    cells_layout(out->cells, out->n_receptors, out->n_atoms, &dst);
+    int r_off = 0, a_off = 0;
+    for (int k = 0; k < n_parts; ++k) {
+        const pvs_pocket *q = parts[k];
+        PocketCells src;
+        cells_layout(q->cells, q->n_receptors, q->n_atoms, &src);
+        const int64_t work = std::max<int64_t>((int64_t)q->n_receptors * (PK_MAX_CELLS + 1),
+                                               (int64_t)q->n_atoms * 8);
+        const int grid = (int)std::min<int64_t>(std::max<int64_t>((work + 255) / 256, 1), 1024);
+        pocket_compose_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(
+            src, q->rr_ptr, q->rr_col, q->n_receptors, q->n_atoms, dst, out->rr_ptr, out->rr_col,
+            r_off, a_off, k == 0);
+        rc = check_launch();
+        if (rc) return rc;
+        r_off += q->n_receptors;
+        a_off += q->n_atoms;
+    }
+    return PVS_OK;
 }
 
 int pvs_pocket_graph_count(const pvs_pocket *pocket, const double *coords,

@@ -34,6 +34,19 @@ from .graph import PackedBatch
 
 _COLUMNS = ('x', 'y', 'z', 'atomic_number', 'types', 'bp')
 
+# Device-crop batches run K1p (screening.Pocket) instead of K1 where it pays
+# (profiles/README.md, "Pocket route of the device-crop loader"; B200, 1000 W):
+# * K1p's graph stage beats K1's from 681 atoms per complex up (1.26x at 681,
+#   7.4x at 5469) and loses below 381 (0.93-0.95x for whole proteins at a
+#   10 A crop around 18-atom ligands), so a batch whose complexes average
+#   fewer atoms than POCKET_MIN_COMPLEX_ATOMS runs K1;
+# * a pocket build takes 0.20-0.23 ms (1754-5450 atoms) and the smallest
+#   saving measured where K1p is chosen is 0.23 us per pose, so a receptor
+#   gets a pocket only when at least POCKET_MIN_POSES poses will use it while
+#   it stays resident.
+POCKET_MIN_COMPLEX_ATOMS = 512
+POCKET_MIN_POSES = 1024
+
 
 # --------------------------------------------------------------------------
 # types files
@@ -447,6 +460,10 @@ class ComplexDataset:
         # filter / typing / one-hot of every pose run on the GPU (K0)
         self.device_crop = bool(device_crop)
         self._rec_dev = OrderedDict()
+        # resident pockets (K1p), keyed as _rec_dev and dropped with it, and
+        # the receptors worth one per upcoming batch (plan_pockets)
+        self._pockets = {}
+        self._pocket_plan = None
         self.use_types = True
         self._rng = np.random.default_rng(seed)
         self._cache = OrderedDict()
@@ -522,6 +539,8 @@ class ComplexDataset:
         state['_cache_lock'] = None
         state['_cache'] = OrderedDict()
         state['_rec_dev'] = OrderedDict()
+        state['_pockets'] = {}
+        state['_pocket_plan'] = None
         state['sampler'] = None
         return state
 
@@ -616,16 +635,83 @@ class ComplexDataset:
         with self._cache_lock:
             self._rec_dev[key] = entry
             while len(self._rec_dev) > max(1, self._cache_size):
-                self._rec_dev.popitem(last=False)
+                gone, _ = self._rec_dev.popitem(last=False)
+                self._pockets.pop(gone, None)
         return entry
 
-    def crop_on_device(self, items, ligands=None):
-        """K0 for the complexes `items`: -> (coords f64 [N,3], bp i32 [N],
-        feats f32 [N,F]) on the device and the host complex_ptr [B+1]."""
-        device = torch.device(self.device or 'cuda')
-        if ligands is None:
-            ligands = [self.load_ligand(i) for i in items]
-        # receptors of this batch, each uploaded once and kept
+    # -- resident pockets (K1p) -----------------------------------------------
+    def plan_pockets(self, batches):
+        """Decide, for the batch sequence `batches` (lists of items, in the
+        order they will be packed), which receptors get a pocket: those that
+        at least POCKET_MIN_POSES poses use while they stay resident.  The
+        residency follows the device receptor LRU (`receptor_cache`) from its
+        present state.  batches=None (a sampled order) builds none."""
+        if batches is None:
+            self._pocket_plan = None
+            return
+        dev = str(torch.device(self.device or 'cuda'))
+        cap = max(1, self._cache_size)
+        lru = OrderedDict((k[0], None) for k in self._rec_dev if k[1] == dev)
+        # residency: [poses, batch keys]; one per receptor upload
+        current, residencies = {}, []
+        for items in batches:
+            names = list(dict.fromkeys(str(self.receptor_fnames[i])
+                                       for i in items))
+            for name in names:
+                if name in lru:
+                    lru.move_to_end(name)
+                else:
+                    lru[name] = None
+                    current.pop(name, None)
+                    while len(lru) > cap:
+                        gone, _ = lru.popitem(last=False)
+                        current.pop(gone, None)
+                if name not in current:
+                    current[name] = [0, []]
+                    residencies.append((name, current[name]))
+                res = current[name]
+                res[0] += sum(1 for i in items
+                              if str(self.receptor_fnames[i]) == name)
+                res[1].append(tuple(items))
+        plan = {}
+        for name, (poses, keys) in residencies:
+            if poses >= POCKET_MIN_POSES:
+                for key in keys:
+                    plan.setdefault(key, set()).add(name)
+        self._pocket_plan = plan
+
+    def pocket_route(self, items, rec_atoms, lig_atoms, complex_atoms):
+        """The graph builder of device-crop batch `items`: -> (use_k1p,
+        names of the receptors whose pocket to build first).
+
+        rec_atoms: atoms of each receptor of the batch (name -> int);
+        lig_atoms: emitted ligand atoms of each pose; complex_atoms: atoms of
+        each complex K0 assembled.  K1p runs when every receptor has a
+        resident pocket for the dataset's radii (or the plan builds it now),
+        every receptor and pose is within K1p's bounds and the complexes
+        average at least POCKET_MIN_COMPLEX_ATOMS atoms; anything else runs
+        K1, which builds the same graph."""
+        from ._cabi import (POCKET_MAX_LIG_ATOMS,   # noqa: PLC0415
+                            POCKET_MAX_REC_ATOMS)
+        if not items or max(lig_atoms) > POCKET_MAX_LIG_ATOMS or \
+                max(rec_atoms.values()) > POCKET_MAX_REC_ATOMS or \
+                np.mean(complex_atoms) < POCKET_MIN_COMPLEX_ATOMS:
+            return False, []
+        dev = str(torch.device(self.device or 'cuda'))
+        radii = (float(self.inter_radius), float(self.intra_radius))
+        planned = (self._pocket_plan or {}).get(tuple(items), ())
+        build = []
+        for name in rec_atoms:
+            have = self._pockets.get((name, dev))
+            if have is not None and have[0] == radii:
+                continue
+            if name not in planned:
+                return False, []
+            build.append(name)
+        return True, build
+
+    def _batch_receptors(self, items):
+        """Receptor names of a batch in first-use order, and rec_of_pose."""
         rec_names, rec_index = [], {}
         rec_of_pose = np.zeros(len(items), dtype=np.int32)
         for b, i in enumerate(items):
@@ -634,9 +720,56 @@ class ComplexDataset:
                 rec_index[name] = len(rec_names)
                 rec_names.append(name)
             rec_of_pose[b] = rec_index[name]
+        return rec_names, rec_of_pose
+
+    def crop_on_device(self, items, ligands=None):
+        """K0 for the complexes `items`: -> (coords f64 [N,3], bp i32 [N],
+        feats f32 [N,F]) on the device and the host complex_ptr [B+1]."""
+        device = torch.device(self.device or 'cuda')
+        if ligands is None:
+            ligands = [self.load_ligand(i) for i in items]
+        # receptors of this batch, each uploaded once and kept
+        rec_names, rec_of_pose = self._batch_receptors(items)
         recs = [self.receptor_on_device(name, device) for name in rec_names]
         return crop_batch(ligands, recs, rec_of_pose, self.radius,
                           self.n_features, self.compact, device)
+
+    def _device_graph(self, items, ligands, edge_capacity):
+        """K0, then K1p or K1 as pocket_route picks, for batch `items` ->
+        (CropOutput, CSRGraph)."""
+        from .graph import radius_graph_batch   # noqa: PLC0415
+        from .screening import Pocket   # noqa: PLC0415
+        device = torch.device(self.device or 'cuda')
+        if ligands is None:
+            ligands = [self.load_ligand(i) for i in items]
+        rec_names, rec_of_pose = self._batch_receptors(items)
+        recs = [self.receptor_on_device(name, device) for name in rec_names]
+        crop = crop_batch_masked(ligands, recs, rec_of_pose, self.radius,
+                                 self.n_features, self.compact, device)
+        cptr_host = crop.complex_ptr_host
+        lig_count = [int(np.count_nonzero(l.emit)) for l in ligands]
+        use, build = self.pocket_route(
+            items, {n: int(r[0].shape[0]) for n, r in zip(rec_names, recs)},
+            lig_count, np.diff(cptr_host))
+        if not use:
+            return crop, radius_graph_batch(
+                crop.coords, crop.bp, cptr_host, self.inter_radius,
+                self.intra_radius, device=device, edge_capacity=edge_capacity)
+        radii = (float(self.inter_radius), float(self.intra_radius))
+        parts = []
+        for name, rec in zip(rec_names, recs):
+            key = (name, str(device))
+            if name in build:
+                parts.append(Pocket(rec, *radii))
+                with self._cache_lock:   # resident with its receptor only
+                    if key in self._rec_dev:
+                        self._pockets[key] = (radii, parts[-1])
+            else:
+                parts.append(self._pockets[key][1])
+        # composed on the caller's stream, which K1p runs on
+        pocket = Pocket.compose(parts)
+        return crop, pocket.radius_graph(crop, lig_count,
+                                         edge_capacity=edge_capacity)
 
     def prepare(self, item):
         """What a loader thread does ahead of the device for one complex."""
@@ -690,11 +823,9 @@ class ComplexDataset:
                             dtype=torch.float32)
 
     def _pack_device(self, items, ligands, edge_capacity):
-        from .graph import radius_graph_batch   # noqa: PLC0415
-        coords, bp, feats, cptr_host = self.crop_on_device(items, ligands)
-        csr = radius_graph_batch(coords, bp, cptr_host, self.inter_radius,
-                                 self.intra_radius, device=coords.device,
-                                 edge_capacity=edge_capacity)
+        crop, csr = self._device_graph(items, ligands, edge_capacity)
+        coords, feats, cptr_host = crop.coords, crop.feats, \
+            crop.complex_ptr_host
         pos = coords.float()
         if self.rot:
             pos_h = coords.cpu().numpy().copy()
@@ -768,6 +899,8 @@ class PackedLoader:
         everything that happens before the device is involved."""
         batches = self._batches()
         ds = self.dataset
+        if ds.device_crop:
+            ds.plan_pockets(batches if self.sampler is None else None)
         if self.num_workers <= 0:
             for items in batches:
                 yield items, [ds.prepare(i) for i in items]

@@ -101,6 +101,55 @@ class Pocket:
             torch.cuda.current_stream(dev).synchronize()
 
     @classmethod
+    def compose(cls, pockets):
+        """One pocket of the receptors of `pockets` (built pockets of the
+        same radii and device), in that order, assembled by device copies:
+        no receptor is searched again.  Runs on the current stream, which
+        must be ordered before any other stream reads the result."""
+        pockets = list(pockets)
+        if len(pockets) == 1:
+            return pockets[0]
+        if not pockets:
+            raise ValueError('a pocket needs at least one receptor')
+        first = pockets[0]
+        for p in pockets[1:]:
+            first.check_radii(p.inter_radius, p.intra_radius)
+        self = cls.__new__(cls)
+        self.inter_radius, self.intra_radius = first.inter_radius, \
+            first.intra_radius
+        self.device = dev = first.device
+        self.receptors = [r for p in pockets for r in p.receptors]
+        sizes = [int(r[0].shape[0]) for r in self.receptors]
+        self.rec_ptr_host = np.zeros(len(sizes) + 1, dtype=np.int32)
+        np.cumsum(sizes, out=self.rec_ptr_host[1:])
+        n_atoms = int(self.rec_ptr_host[-1])
+        self.n_rr_edges = sum(p.n_rr_edges for p in pockets)
+        h = lib()
+        with torch.cuda.device(dev):
+            self.xyz = torch.cat([p.xyz for p in pockets])
+            self.emit = torch.cat([p.emit for p in pockets])
+            self.code = torch.cat([p.code.to(torch.int16) for p in pockets])
+            self.rec_ptr = torch.from_numpy(self.rec_ptr_host.copy()).to(dev)
+            self.cells = torch.empty(
+                max(256, int(h.pvs_pocket_cells_bytes(len(sizes), n_atoms))),
+                dtype=torch.uint8, device=dev)
+            self.rr_ptr = torch.empty(n_atoms + 1, dtype=torch.int32,
+                                      device=dev)
+            self.rr_col = torch.empty(max(1, self.n_rr_edges),
+                                      dtype=torch.int32, device=dev)
+            self.desc = _cabi.PocketDesc(
+                len(sizes), n_atoms, max(sizes), self.inter_radius,
+                self.intra_radius, ptr(self.xyz), ptr(self.emit),
+                ptr(self.rec_ptr), ptr(self.cells), ptr(self.rr_ptr),
+                ptr(self.rr_col))
+            parts = (C.POINTER(_cabi.PocketDesc) * len(pockets))(
+                *[C.pointer(p.desc) for p in pockets])
+            check(h.pvs_pocket_compose(parts, len(pockets),
+                                       C.byref(self.desc), stream()),
+                  'pvs_pocket_compose')
+        return self
+
+    @classmethod
     def from_dataset(cls, dataset, rec_fnames, device=None):
         """Pocket of `dataset`'s receptors `rec_fnames` (one name or a list)
         at the dataset's edge radii."""
